@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA path through the C ABI)
   python bench.py --impl reference --gpus N --steps K ...  the reference's own CPU path (oracle/_ref)
+  python bench.py ... --dump-outputs DIR                   also write the last timed step's results to DIR/*.npy
 
 A step = one full log-likelihood evaluation (`ProbCalculator::CalcProb` on a fresh ScoringState,
 prob_calculator.h:63-109).
@@ -24,6 +25,7 @@ evaluations of the annealing loop are reported beside it as `sa_iters_per_s`.
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -113,6 +115,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "100",
                                           "-i", str(self.device)], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)   # a run that fails before stop() must not leave the poller running
             self.thread = threading.Thread(target=self._read, daemon=True)
             self.thread.start()
         except Exception:
@@ -141,6 +144,27 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_READ_VALUES_MAX = 1 << 21   # every read of config 2 (2 M pairs); a larger shard is sampled
+
+
+def dump_outputs(out_dir: str, pc, gathered, total_len: int, world: int) -> None:
+    """Writes what the timed evaluation returned in its last step, as float64 .npy files: the partial sums of every rank
+    (`partials`), their exact combination (`prob`, `floored` = [set][floored reads, reads], `total_len`) and the per-read
+    values of this rank's first read set (`read_values`; for a set of more than DUMP_READ_VALUES_MAX reads a fixed, seeded
+    sample of them, whose read indices go to `read_index`)."""
+    os.makedirs(out_dir, exist_ok=True)
+    prob, zeros, tl = pc.combine(gathered, world, total_len)
+    arrays = {"partials": gathered, "prob": [prob], "floored": zeros, "total_len": [tl]}
+    values = pc.read_values(0)
+    if len(values) > DUMP_READ_VALUES_MAX:
+        idx = np.sort(np.random.default_rng(0).choice(len(values), DUMP_READ_VALUES_MAX, replace=False))
+        values = values[idx]
+        arrays["read_index"] = idx
+    arrays["read_values"] = values
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def measured_peak():
@@ -323,7 +347,15 @@ def main():
     ap.add_argument("--exchange", default="host", choices=["peer", "host", "nccl"],
                     help="how the ranks' result lines meet (N > 1): host shared memory written by the kernels (default: the fastest end to "
                          "end on the 8-GPU box, profiles/r02_exchange_ab.md), NVLink peer memory, ncclAllReduce")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed evaluation to DIR/<name>.npy, so that two builds can be compared "
+                         "output for output: all ranks' partial sums and their combination, rank 0's per-read values of its "
+                         "first read set (CUDA arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "gaml_b200":
+        ap.error("--dump-outputs needs --impl gaml_b200: the reference arm reports timings only")
     args.warmup = max(args.warmup, 3) if args.impl == "gaml_b200" else args.warmup
 
     if args.impl == "reference":
@@ -486,6 +518,8 @@ def main():
     st = pc.stats()
     launches = st.kernel_launches - launches0
     a_local, bytes_local = st.last_records_gathered, st.last_algorithmic_bytes
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pc, g_full, tl, world)
     # roofline timing of the streaming pass: the same steps again with the library's per-kernel events switched on
     # (an event between two kernels serialises them, so the chained launches of the timed region above are given up
     # at the two boundaries of the streaming pass; the kernels themselves are identical)

@@ -48,11 +48,3 @@ def oracle(tmp_path):
     def _run(wl, name="case", dump=True):
         return run_scorer(ORACLE_BIN, wl, tmp_path, name, dump)
     return _run
-
-
-def has_gpu() -> bool:
-    try:
-        import torch
-        return torch.cuda.is_available()
-    except Exception:
-        return False

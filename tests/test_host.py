@@ -9,7 +9,7 @@ import sys
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, ROOT, has_gpu
+from conftest import GOLDEN, ROOT
 from gaml_b200 import api, dist, synth, workload
 
 
@@ -29,11 +29,18 @@ def test_struct_layouts_match_header():
     assert workload.ALN_DTYPE.itemsize == 16 and workload.PB_DTYPE.itemsize == 24
 
 
-@pytest.mark.skipif(has_gpu(), reason="checks the no-GPU failure mode")
 def test_no_cpu_fallback_without_gpu():
-    with pytest.raises(api.GamlError) as ei:
-        api.ProbCalculator([100, 100])
-    assert "no CPU fallback" in str(ei.value)
+    """Run in a child process that sees no CUDA device, so that the no-GPU failure mode is checked on GPU machines too."""
+    code = ("import sys; sys.path.insert(0, {root!r})\n"
+            "from gaml_b200 import api\n"
+            "try:\n"
+            "    api.ProbCalculator([100, 100])\n"
+            "except api.GamlError as e:\n"
+            "    print('GamlError:', e)\n").format(root=ROOT)
+    out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True,
+                         text=True, timeout=120)
+    assert out.returncode == 0, out.stdout + out.stderr
+    assert out.stdout.startswith("GamlError:") and "no CPU fallback" in out.stdout, out.stdout
 
 
 def test_combine_raw_is_pure_host_arithmetic():
