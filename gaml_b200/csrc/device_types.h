@@ -153,7 +153,8 @@ struct ScoreParams {
   int32_t n_mtouch, n_mtouch1;
   // chain discipline of the streaming kernels (set per launch)
   int32_t chain_first;       // 1: first kernel after apply_slots in its group: waits at its top; 0: waits at its end
-  int32_t finish_here;       // 1: this kernel's last block publishes the set when nothing was listed for the pass after it
+  int32_t finish_here;       // 1: this kernel's last block publishes the set when nothing was listed for the pass after it;
+                             // 2: no pass follows: it publishes the set, as a pending line when reads were listed
   uint32_t* tile_counter;    // next tile of [0] tier 1, [1] the rare shapes, [2] tier 2, [3] the cross list, then the appendix (zeroed by apply_slots)
   uint32_t* ticket2;         // blocks-finished counter of the set's last kernel (finish_set)
   uint32_t* done;            // set by finish_set_if_complete

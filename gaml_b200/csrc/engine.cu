@@ -241,6 +241,13 @@ struct ReadSetState {
   std::vector<uint32_t> h_pb_prefix;
   std::vector<int> h_pb_walk_len;
   std::vector<int> h_bad;
+  // paired full evaluations replayed as a graph end with the streaming kernel unless the set's previous full evaluation
+  // listed reads for the many-placement pass (keep_tail). Without the pass in the chain, a pending line makes finish()
+  // run it on demand with the parameters kept here.
+  bool keep_tail = false;
+  bool tail_on_demand = false;  // the pending evaluation's chain has no many-placement pass
+  ScoreParams tail_params{};
+  int tail_grid = 0;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // around this set's streaming kernel(s)
   ~ReadSetState() {
     for (cudaEvent_t e : {ev0, ev1})
@@ -367,6 +374,7 @@ struct gaml_ctx {
   bool use_graphs = true;
   bool running_total = true;      // GAML_B200_NO_RUNNING_TOTAL=1 forces the O(R) pass on every incremental evaluation (tests)
   bool timing_pending = false;    // events of the last evaluation not yet turned into gaml_stats times
+  bool tail_timed = false;        // finish() ran many-placement passes on demand between ev[1] and ev[2] (timed)
   size_t h_out_cap = 0;
   unsigned long long scratch_entries = 1ull << 22;   // 4 Mi placements (96 MiB) for many-placement reads
   uint32_t ovf_cap = 1u << 20;
@@ -2128,7 +2136,11 @@ int launch(gaml_ctx* ctx) {
   char* blob = ctx->blob_dev;
   int launches = 0;
   bool any_penalty = false;
-  for (auto& rs : ctx->sets) any_penalty |= rs->penalty || rs->pb_penalty;
+  for (auto& rs : ctx->sets) {
+    any_penalty |= rs->penalty || rs->pb_penalty;
+    rs->tail_on_demand = false;
+  }
+  ctx->tail_timed = false;
   LaunchList chain;
   const bool record = ctx->use_graphs && !ctx->profile && !any_penalty && ctx->sets.size() <= 3;
   struct RecorderGuard { ~RecorderGuard() { set_launch_recorder(nullptr); } } recorder_guard;
@@ -2169,7 +2181,15 @@ int launch(gaml_ctx* ctx) {
     if (rs.cfg.kind == GAML_KIND_PAIRED) {
       if (sp.full) {
         const uint32_t n_multi = (uint32_t)sp.multi_records;
-        launches += launch_paired_full(P, sp.grid, sp.cgrid, n_multi, og, ctx->sm_count, st, chained, profile, rs.ev0, rs.ev1);
+        // the streaming kernel ends a graph-replayed chain whose line only this host waits for first: the host segment
+        // exchange (or none) — the peer and collective exchanges consume the line on the device
+        rs.tail_on_demand = record && !ctx->peer_on && !nccl_lines(ctx) && !rs.keep_tail;
+        if (rs.tail_on_demand) {
+          rs.tail_params = P;
+          rs.tail_grid = og;
+        }
+        launches += launch_paired_full(P, sp.grid, sp.cgrid, n_multi, og, ctx->sm_count, st, chained, profile, rs.ev0, rs.ev1,
+                                       !rs.tail_on_demand);
         any_full = true;
         // DESIGN.md §4: 16 B per live record + packed lengths (4) + probs write (8) per pair (no probs read: fused)
         bytes += 16 * sp.records + 12 * (int64_t)rs.n_local;
@@ -2268,8 +2288,10 @@ int launch(gaml_ctx* ctx) {
   return GAML_OK;
 }
 
-// Waits for one 64-byte result line of this evaluation (flag word = epoch, checksum intact) and copies it out.
-int wait_line(gaml_ctx* ctx, const volatile uint64_t* line, uint64_t want_bits, double* dst, bool own) {
+// Waits for one 64-byte result line of this evaluation (flag word = epoch, checksum intact) and copies it out. With
+// `pending`, a line whose flag word is pend_bits is accepted too, and *pending tells which of the two arrived.
+int wait_line(gaml_ctx* ctx, const volatile uint64_t* line, uint64_t want_bits, double* dst, bool own, bool* pending = nullptr,
+              uint64_t pend_bits = 0) {
   unsigned spins = 0;
   const auto t0 = std::chrono::steady_clock::now();
   for (;;) {
@@ -2277,8 +2299,10 @@ int wait_line(gaml_ctx* ctx, const volatile uint64_t* line, uint64_t want_bits, 
     for (int j = 0; j < 8; j++) w[j] = line[j];
     uint64_t sum = kResultSeal;
     for (int j = 0; j < 7; j++) sum ^= w[j];
-    if (w[6] == want_bits && w[7] == sum) {
+    const bool alt = pending && w[6] == pend_bits;
+    if ((w[6] == want_bits || alt) && w[7] == sum) {
       memcpy(dst, w, sizeof(w));
+      if (pending) *pending = alt;
       return GAML_OK;
     }
     cpu_relax();
@@ -2355,10 +2379,38 @@ int finish(gaml_ctx* ctx, double* partials, int32_t* total_len, double* gathered
     // polled now and then so that a failed launch surfaces as an error instead of a hang.
     // A line counts only when its flag word carries this evaluation's epoch AND its checksum matches: the device
     // writes all eight words with one store and no fence, so a partially arrived line must be told from a whole one.
+    // A set whose chain ended with its streaming kernel may instead publish a pending line (flag word -epoch): it listed
+    // reads for the many-placement pass, which runs now, on demand, and publishes the final line.
     const volatile uint64_t* ho = reinterpret_cast<const volatile uint64_t*>(own_lines);
+    const double pend_d = -(double)ctx->epoch;
+    uint64_t pend_bits;
+    memcpy(&pend_bits, &pend_d, 8);
+    bool any_pending = false;
     for (size_t s = 0; s < n_sets; s++) {
-      const int rc = wait_line(ctx, ho + s * kResultStride, want_bits, ctx->h_res.data() + s * kResultStride, true);
+      ReadSetState& rs = *ctx->sets[s];
+      bool pending = false;
+      const int rc = wait_line(ctx, ho + s * kResultStride, want_bits, ctx->h_res.data() + s * kResultStride, true,
+                               rs.tail_on_demand ? &pending : nullptr, pend_bits);
       if (rc != GAML_OK) return rc;
+      if (!pending) continue;
+      if (!any_pending && ctx->timed) CU(cudaEventRecord(ctx->ev[1], ctx->stream));
+      any_pending = true;
+      launch_paired_tail(rs.tail_params, rs.tail_grid, ctx->stream);
+      CU(cudaGetLastError());
+      ctx->stats.kernel_launches++;
+    }
+    if (any_pending) {
+      if (ctx->timed) {
+        CU(cudaEventRecord(ctx->ev[2], ctx->stream));
+        ctx->tail_timed = true;
+      }
+      for (size_t s = 0; s < n_sets; s++) {
+        uint64_t flag;
+        memcpy(&flag, ctx->h_res.data() + s * kResultStride + 6, 8);
+        if (!ctx->sets[s]->tail_on_demand || flag != pend_bits) continue;
+        const int rc = wait_line(ctx, ho + s * kResultStride, want_bits, ctx->h_res.data() + s * kResultStride, true);
+        if (rc != GAML_OK) return rc;
+      }
     }
     std::atomic_thread_fence(std::memory_order_acquire);
   }
@@ -2412,6 +2464,7 @@ int finish(gaml_ctx* ctx, double* partials, int32_t* total_len, double* gathered
     scratch_placements = std::max<int64_t>(scratch_placements, (int64_t)(f >> 28));
     if (rs.pb_penalty && !rs.sharded) rs.bad_bases = rs.h_bad[0];
     if (rs.cfg.kind == GAML_KIND_PAIRED) {
+      if (ctx->plan[s].full) rs.keep_tail = ((f >> 4) & 0xffffff) != 0;   // expected to list reads again next time
       if (rs.penalty && !rs.sharded) {   // EraseFromScoringState / AddToScoringState, graph.cc:1938, 1946
         if (ctx->plan[s].full) rs.bad_bases = 0;
         for (int w = 0; w < ctx->plan[s].n_cov_walks; w++)
@@ -3980,6 +4033,11 @@ int gaml_get_stats(gaml_ctx* ctx, gaml_stats* out) {
     cudaSetDevice(ctx->device);
     float ms = 0, ms2 = 0;
     if (cudaEventSynchronize(ctx->ev[3]) == cudaSuccess) cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[3]);
+    if (ctx->tail_timed) {   // + the many-placement passes finish() ran on demand after the chain
+      float t = 0;
+      if (cudaEventSynchronize(ctx->ev[2]) == cudaSuccess && cudaEventElapsedTime(&t, ctx->ev[1], ctx->ev[2]) == cudaSuccess) ms += t;
+      ctx->tail_timed = false;
+    }
     if (ctx->profile)
       for (auto& rs : ctx->sets) {
         float t = 0;

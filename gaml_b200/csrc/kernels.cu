@@ -171,17 +171,21 @@ struct PublishArgs {
   int32_t peer_world;
   uint32_t peer_line;
   double* part_out;
+  int32_t last_in_chain;   // the streaming kernel ends the chain (finish_here 2): listed reads give a pending line
 };
 __device__ __forceinline__ PublishArgs publish_args(const ScoreParams& P, uint32_t* ticket) {
   return PublishArgs{P.accum, P.state_acc, P.out, P.error_flag, P.ovf_count, P.scratch_cursor, ticket, P.done, P.epoch, P.state_add,
-                     P.ql, (long long)P.n_reads, P.peer_bufs, P.peer_world, P.peer_line, P.part_out};
+                     P.ql, (long long)P.n_reads, P.peer_bufs, P.peer_world, P.peer_line, P.part_out, P.finish_here == 2};
 }
 
 // Called by the first warp of the completing block. Lane 0 assembles the eight result words; lanes 0..7 then store
 // one word each with ONE instruction — a single 64-byte write to the host instead of eight, and no system-wide fence
 // between payload and flag: word 6 is the evaluation's epoch (the flag the host spins on) and word 7 a checksum of
 // the other seven, so the host accepts the line only when it is complete, whatever order its bytes arrive in.
-__device__ __noinline__ void publish_set(PublishArgs A) {
+// pending: the set still owes the terms of the reads listed for the many-placement pass, which the owning host runs
+// on demand. Word 6 is then -epoch, which no host waiting for the final line accepts, and the running total is left
+// alone (that pass commits it).
+__device__ __noinline__ void publish_set(PublishArgs A, bool pending) {
   const int lane = threadIdx.x & 31;
   unsigned long long w[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   if (lane == 0) {
@@ -190,7 +194,7 @@ __device__ __noinline__ void publish_set(PublishArgs A) {
     for (int j = 0; j < 7; j++) a[j] = __ldcg(A.accum + j);
     unsigned __int128 x = 0;
     for (int j = 0; j < 4; j++) x += (unsigned __int128)a[j] << (32 * j);
-    if (A.state_acc) {
+    if (A.state_acc && !pending) {
       // paired sets keep their running total {low, high 64 bits, floored, -inf, nan} on the device: a delta-only
       // evaluation accumulated (new term - old term) of the touched reads and adds it, any other sets it
       if (A.state_add) {
@@ -215,7 +219,7 @@ __device__ __noinline__ void publish_set(PublishArgs A) {
     // flags: error bits (4) | listed reads (24 bits) | scratch placements (24 bits, saturating)
     w[5] = (unsigned long long)__double_as_longlong((double)__ldcg(A.error_flag) + 16.0 * (double)min(__ldcg(A.ovf_count), 0xffffffu) +
                                                     268435456.0 * (double)min(scratch, 0xffffffull));
-    w[6] = (unsigned long long)__double_as_longlong((double)A.epoch);
+    w[6] = (unsigned long long)__double_as_longlong(pending ? -(double)A.epoch : (double)A.epoch);
     w[7] = kResultSeal;
     for (int j = 0; j < 7; j++) w[7] ^= w[j];
   }
@@ -298,22 +302,28 @@ __global__ void reduced_publish_kernel(const double* reduced, int n_sets, uint32
 // draws the final ticket publishes. early = true: called by every block of the set's last STREAMING kernel
 // (P.finish_here): if no read was listed for the many-placement pass, the last block publishes right away and marks the
 // set done — the pass that follows in the chain then has nothing to do, and the host has its result one kernel earlier.
+// When no pass follows (A.last_in_chain) and reads were listed, the last block publishes a pending line instead: the
+// owning host then runs the many-placement pass, which publishes the final one.
 __device__ __noinline__ void finish_blocks(PublishArgs A, bool early) {
-  __shared__ bool s_last;
+  __shared__ bool s_last, s_pending;
   __threadfence();
   __syncthreads();
   if (threadIdx.x == 0) {
     bool last = atomicAdd(A.ticket, 1u) == gridDim.x - 1;
+    bool pending = false;
     if (last && early) {
       __threadfence();
-      last = __ldcg(A.ovf_count) == 0;
+      pending = __ldcg(A.ovf_count) != 0;
+      last = !pending || A.last_in_chain;
     }
     s_last = last;
+    s_pending = pending;
   }
   __syncthreads();
   if (!s_last || threadIdx.x >= 32) return;
-  publish_set(A);
-  if (early && threadIdx.x == 0) *A.done = 1u;
+  const bool pending = s_pending;
+  publish_set(A, pending);
+  if (early && !pending && threadIdx.x == 0) *A.done = 1u;
 }
 __device__ __forceinline__ void finish_set(const ScoreParams& P) { finish_blocks(publish_args(P, P.ticket2), false); }
 __device__ __forceinline__ void finish_set_if_complete(const ScoreParams& P) { finish_blocks(publish_args(P, P.ticket), true); }
@@ -1789,7 +1799,8 @@ __global__ void __launch_bounds__(kOvfBlock) paired_delta_kernel(const ScorePara
 // Many-placement pass: the reads the streaming / delta kernel listed because they need the enumeration order.
 // full_mode 1: full evaluation (state from 0, terms summed, per-set finalize); 0: delta followed by the O(R) total pass;
 // 2: delta-only evaluation (new term - old term into the running total, per-set finalize). In modes 1 and 2 the kernel
-// before it has already published the set when it listed nothing (P.done).
+// before it has already published the set when it listed nothing (P.done). Mode 1 also runs on its own, submitted by the
+// host after a chain without it ended with a pending line (launch_paired_tail).
 __global__ void __launch_bounds__(kOvfBlock) paired_overflow_kernel(const ScoreParams P, int full_mode) {
   tl_begin(P.timeline, kTlOverflow);
   pdl_release();
@@ -3009,15 +3020,19 @@ void launch_apply_slots(const SlotUpdate* upd, int n, const SlotUpdate* patch, i
 // wait for the first in the ordinary way, so profiling costs the overlap at those two boundaries.
 // Tier 1 and tier 2 touch disjoint reads and only meet in the (commutative, integer) accumulators.
 int launch_paired_full(const ScoreParams& P, int grid, int cgrid, uint32_t n_multi_items, int ovf_grid, int sm_count,
-                       cudaStream_t st, bool chained, bool profile, cudaEvent_t e0, cudaEvent_t e1) {
+                       cudaStream_t st, bool chained, bool profile, cudaEvent_t e0, cudaEvent_t e1, bool tail) {
   int n_launched = 0;
-  // chain: [multi pass] -> streaming kernel (tier 1 + tier 2) -> many-placement pass. Only two kernels of a chain are in
+  // chain: [multi pass] -> streaming kernel (tier 1 + tier 2) [-> many-placement pass]. Without the trailing pass (!tail)
+  // the streaming kernel ends the chain: it publishes the final line when it listed no read, else a pending one, and
+  // the owning host runs the pass on demand (launch_paired_tail). The trailing pass would otherwise wait with 148
+  // register-hungry blocks that cannot become resident before streaming blocks retire. Only two kernels of a chain are in
   // flight at a time (kernel n+2 starts when kernel n has completed), so the multi pass — a small grid of
   // register-hungry blocks with a long dependent chain, needing apply_slots only — goes FIRST and runs underneath the
   // streaming kernel, whose tile counters absorb the register file it holds meanwhile. It waits for apply_slots at its
   // top and releases after; the streaming kernel then starts without waiting and waits at its END, which makes
   // completion transitive for the last kernel. (cgrid is unused here: tier 2 is a phase of the streaming kernel.)
   (void)cgrid;
+  tail = tail || profile;
   ScoreParams Q = P;
   bool dep = chained && !profile;
   bool first = true;
@@ -3035,7 +3050,7 @@ int launch_paired_full(const ScoreParams& P, int grid, int cgrid, uint32_t n_mul
   }
   if (profile) cudaEventRecord(e0, st);
   Q.chain_first = first || profile ? 1 : 0;
-  Q.finish_here = profile ? 0 : 1;   // when profiling, e0/e1 bracket the streaming work alone: the last kernel publishes
+  Q.finish_here = profile ? 0 : (tail ? 1 : 2);   // when profiling, e0/e1 bracket the streaming work alone: the last kernel publishes
   {
     // one resident wave of the instantiation that runs (its blocks draw tiles from counters)
     static StreamKernel seen[16];
@@ -3068,8 +3083,13 @@ int launch_paired_full(const ScoreParams& P, int grid, int cgrid, uint32_t n_mul
     }
   }
   if (profile) cudaEventRecord(e1, st);
+  if (!tail) return n_launched;
   launch_chain(paired_overflow_kernel, ovf_grid, kOvfBlock, st, !profile, P, 1);
   return n_launched + 1;
+}
+
+void launch_paired_tail(const ScoreParams& P, int ovf_grid, cudaStream_t st) {
+  launch_chain(paired_overflow_kernel, ovf_grid, kOvfBlock, st, false, P, 1);
 }
 
 void launch_paired_delta(const ScoreParams& P, uint32_t n_touch_records, int grid_total, int ovf_grid, int sm_count,

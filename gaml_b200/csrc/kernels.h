@@ -48,8 +48,13 @@ constexpr int kTimelineWords = 12;   // profiling level 2: {start, end} ns of ap
 // launches, kernels.cu): streaming pass (tier 1, tier 2), many-placement pass, per-set finalize in the last block.
 // chained: the operation before it on `st` is a kernel of the chain. profile: record e0 / e1 around the streaming
 // kernel(s) of the set (the roofline timing) — which serialises those two boundaries in the ordinary way.
+// tail: append the many-placement pass (always when profiling). Without it the streaming kernel publishes a pending
+// line (word 6 = -epoch, running total not committed) when it listed reads, and the host calls launch_paired_tail.
 int launch_paired_full(const ScoreParams& P, int grid, int cgrid, uint32_t n_multi_items, int ovf_grid, int sm_count,
-                       cudaStream_t st, bool chained, bool profile, cudaEvent_t e0, cudaEvent_t e1);   // returns the kernels launched
+                       cudaStream_t st, bool chained, bool profile, cudaEvent_t e0, cudaEvent_t e1,
+                       bool tail);   // returns the kernels launched
+// The many-placement pass of a full evaluation whose chain ended with a pending line: publishes the final line.
+void launch_paired_tail(const ScoreParams& P, int ovf_grid, cudaStream_t st);
 void launch_paired_delta(const ScoreParams& P, uint32_t n_touch_records, int grid_total, int ovf_grid, int sm_count, cudaStream_t st,
                          bool chained, bool profile, cudaEvent_t e0, cudaEvent_t e1);
 void launch_single_full(const ScoreParams& P, int grid, int cgrid, int ovf_grid, cudaStream_t st, bool chained, bool profile,
