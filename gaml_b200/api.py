@@ -47,7 +47,8 @@ class Stats(C.Structure):
                 ("last_launch_host_us", C.c_double), ("last_finish_host_us", C.c_double),
                 ("last_scratch_placements", C.c_int64), ("last_multi_items", C.c_int64),
                 ("fast_change_evals", C.c_int64), ("delta_only_evals", C.c_int64), ("cache_appends", C.c_int64),
-                ("cache_rebuilds", C.c_int64), ("full_reuse_evals", C.c_int64), ("full_patch_evals", C.c_int64)]
+                ("cache_rebuilds", C.c_int64), ("full_reuse_evals", C.c_int64), ("full_patch_evals", C.c_int64),
+                ("last_batch_cov_events", C.c_int64), ("last_batch_cov_segments", C.c_int64)]
 
 
 EXPORTS = ["gaml_ctx_create", "gaml_ctx_destroy", "gaml_last_error", "gaml_ctx_stream", "gaml_set_graph",
@@ -383,7 +384,8 @@ class ProbCalculator:
         return probs, tls
 
     def calc_prob_batch(self, candidates):
-        """candidates: list of (erased base-walk indices, added walks). -> (probs [n], total_lens [n], zeros [n][sets])."""
+        """candidates: list of (erased base-walk indices, added walks). -> (probs [n], total_lens [n], zeros [n][sets]).
+        Paired sets only; a penalised set is scored with each candidate's own coverage-gap bad bases."""
         n = len(candidates)
         er_off = np.zeros(n + 1, dtype=np.int64)
         ca_off = np.zeros(n + 1, dtype=np.int64)

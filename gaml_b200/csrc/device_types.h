@@ -263,6 +263,9 @@ struct BatchParams {
   unsigned long long* accum_len;    // n_len x kAccumStride: {low, high 64 bits of the exact sum of all reads' FIX terms at that
                                     // length (before the - n FIX(log 2L) part), floored, -inf, nan}
   long long* accum_cand;            // n_cand x 4: {sum of low 32 bits, sum of high 32 bits (signed) of the term deltas, floored delta, bad}
+  // penalised sets: each candidate's first coverage segment (one segment per erased or added walk of a candidate, batch-wide
+  // ids: the candidate's walk ordinal k emits its events under seg_begin[c] + k), or null
+  const int32_t* seg_begin;
 };
 
 }  // namespace gaml

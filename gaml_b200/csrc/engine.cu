@@ -2576,7 +2576,9 @@ int combine_raw(const double* gathered, int n_shards, int n_sets, const int32_t*
   return GAML_OK;
 }
 
-int combine(gaml_ctx* ctx, const double* gathered, int n_shards, int total_len, gaml_result* result, int32_t* zeros) {
+// bad_bases: per set, the coverage-gap bad bases the result is penalised with (a batch candidate's); null: the sets' state
+int combine(gaml_ctx* ctx, const double* gathered, int n_shards, int total_len, gaml_result* result, int32_t* zeros,
+            const int32_t* bad_bases = nullptr) {
   const size_t n_sets = ctx->sets.size();
   for (auto& rs : ctx->sets)
     if (rs->penalty_pending)
@@ -2589,7 +2591,7 @@ int combine(gaml_ctx* ctx, const double* gathered, int n_shards, int total_len, 
     kinds[s] = ctx->sets[s]->cfg.kind;
     counts[s] = ctx->sets[s]->n_total;
     weights[s] = ctx->sets[s]->cfg.weight;
-    pen[s] = ctx->sets[s]->bad_bases * ctx->sets[s]->cfg.penalty_constant;   // int * double like the reference
+    pen[s] = (bad_bases ? bad_bases[s] : ctx->sets[s]->bad_bases) * ctx->sets[s]->cfg.penalty_constant;   // int * double like the reference
   }
   int rc = combine_raw(gathered, n_shards, (int)n_sets, kinds.data(), counts.data(), weights.data(), total_len, result, zeros,
                        pen.data());
@@ -2600,9 +2602,13 @@ int combine(gaml_ctx* ctx, const double* gathered, int n_shards, int total_len, 
 // ---- batched candidate evaluation (BASELINE config 5) ------------------------------------------------------
 // Candidate c = the last evaluated walk set with walks erased_idx[c] removed and its added walks appended. Host
 // work is O(#nodes of the touched walks) per candidate plus O(#base walks) once per batch.
+// bad_bases (n_cand x n_sets, optional): every candidate's coverage-gap bad bases per set. Sets with penalty_constant != 0
+// are scored only when it is given (unsharded contexts: gaml_calc_prob_batch), because the partials alone carry no bad
+// bases: bad_bases_c = the state's - sum over the erased walks + sum over the added walks of the walk's own sweep over the
+// current cache (EraseFromScoringState / AddToScoringState, graph.cc:1938, 1946), one coverage segment per such walk.
 int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx, const int64_t* erased_off,
                             const int32_t* added_nodes, const int64_t* added_walk_off, const int64_t* cand_added_off,
-                            double* partials, int32_t* total_lens, bool reduce_over_ranks = false) {
+                            double* partials, int32_t* total_lens, bool reduce_over_ranks = false, int32_t* bad_bases = nullptr) {
   if (n_cand <= 0 || !erased_off || !cand_added_off || !added_walk_off || !partials)
     return fail(ctx, GAML_ERR_ARG, "bad batch arguments");
   const auto t_batch0 = std::chrono::steady_clock::now();
@@ -2615,7 +2621,13 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
       return fail(ctx, GAML_ERR_UNSUPPORTED, "gaml_calc_prob_batch supports paired read sets only (single / pacbio sets keep no "
                                              "incremental state: every candidate would be a full evaluation)");
     if (!rs->has_state) return fail(ctx, GAML_ERR_STATE, "gaml_calc_prob_batch needs a base state: call gaml_calc_prob first");
-    if (rs->penalty) return fail(ctx, GAML_ERR_UNSUPPORTED, "gaml_calc_prob_batch with penalty_constant != 0 is not supported yet");
+    if (rs->penalty && reduce_over_ranks)
+      return fail(ctx, GAML_ERR_UNSUPPORTED, "gaml_calc_prob_batch_gathered with penalty_constant != 0 is not supported: every "
+                                             "candidate's coverage events would have to be all-gathered over the read-id shards");
+    if (rs->penalty && !bad_bases)
+      return fail(ctx, GAML_ERR_UNSUPPORTED, "gaml_calc_prob_batch_partial with penalty_constant != 0 is not supported: the partials "
+                                             "carry no bad bases, so gaml_combine_partials would apply the base state's value "
+                                             "(use gaml_calc_prob_batch)");
   }
   int rc = commit(ctx);
   if (rc != GAML_OK) return rc;
@@ -2701,6 +2713,7 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
   for (size_t j = 0; j < two_lens.size(); j++) ql[j] = fix_log_host((double)two_lens[j]);
   const int n_len = (int)two_lens.size();
   ctx->h_batch_out.assign((size_t)n_cand * kOutStride, 0.0);
+  ctx->stats.last_batch_cov_events = ctx->stats.last_batch_cov_segments = 0;
   cudaStream_t st = ctx->stream;
 
   for (size_t s = 0; s < n_sets; s++) {
@@ -2714,15 +2727,38 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
     std::vector<uint32_t> range_prefix(1, 0);
     std::vector<int32_t> range_cand;
     uint64_t touch_total = 0;
+    // coverage segments of a penalised set: one per (candidate, erased or added walk), ids in candidate order; per segment
+    // its contig starts (type-1 events, like an incremental evaluation's walks)
+    const bool cov = rs.penalty;
+    std::vector<int32_t> seg_begin, cs_begin(1, 0), cs;
+    std::vector<unsigned long long> type1;
+    uint64_t records1 = 0;
+    std::vector<int> starts;
+    auto add_segment = [&]() {
+      const uint32_t seg = (uint32_t)(cs_begin.size() - 1);
+      for (int p : starts) {
+        type1.push_back(((unsigned long long)seg << 33) | ((unsigned long long)((uint32_t)p ^ 0x80000000u) << 1));
+        cs.push_back(p);
+      }
+      cs_begin.push_back((int32_t)cs.size());
+    };
     for (int c = 0; c < n_cand; c++) {
       OccBuilder obs[2];
       OccBuilder* ob[2] = {&obs[0], &obs[1]};
       SetPlan sp;
       std::vector<TouchRange> touch;
       int ord = 0;
-      for (int bi : cand_erased[c]) flatten_paired_walk(ctx, rs, base_set.view(bi), ord++, ob, sp, &touch);
-      for (const Walk& w : cand_added[c])
-        flatten_paired_walk(ctx, rs, WalkView{w.data(), (int)w.size(), hash_walk(w), -1}, ord++, ob, sp, &touch);
+      if (cov) seg_begin.push_back((int32_t)(cs_begin.size() - 1));
+      for (int bi : cand_erased[c]) {
+        flatten_paired_walk(ctx, rs, base_set.view(bi), ord++, ob, sp, &touch, cov ? &starts : nullptr);
+        if (cov) add_segment();
+      }
+      for (const Walk& w : cand_added[c]) {
+        flatten_paired_walk(ctx, rs, WalkView{w.data(), (int)w.size(), hash_walk(w), -1}, ord++, ob, sp, &touch,
+                            cov ? &starts : nullptr);
+        if (cov) add_segment();
+      }
+      records1 += sp.records1;
       BatchCand& cd = cands[c];
       cd.n_erased = (int)cand_erased[c].size();
       cd.len_index = cand_len_index[c];
@@ -2793,6 +2829,15 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
     const size_t o_qcls = place(qthr_cls.size() * 8);
     const size_t o_lcls = place(len_class.size() * 4);
     const size_t o_ql = place(ql.size() * 8);
+    const size_t n_seg = cs_begin.size() - 1;
+    // event buffer: the type-1 keys, then up to 4 events per touched mate-1 record (the incremental evaluation's rule)
+    const uint64_t ev_cap = cov ? (uint64_t)type1.size() + 4ull * records1 + 4096ull : 0;
+    if (n_seg > 0x7fffffffull || ev_cap > 0x7fffffffull)
+      return fail(ctx, GAML_ERR_CAPACITY, "too many coverage segments or events for one batch");
+    const size_t o_segb = place(seg_begin.size() * 4);
+    const size_t o_csb = place(cs_begin.size() * 4);
+    const size_t o_cs = place(cs.size() * 4);
+    const size_t o_evc = place(4);   // the running event count (starts after the type-1 keys)
     std::vector<char> blob(std::max<size_t>(off, 16));
     auto put = [&](size_t o, const void* p, size_t bytes) { if (bytes) memcpy(blob.data() + o, p, bytes); };
     put(o_cands, cands.data(), cands.size() * sizeof(BatchCand));
@@ -2810,6 +2855,11 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
     put(o_qcls, qthr_cls.data(), qthr_cls.size() * 8);
     put(o_lcls, len_class.data(), len_class.size() * 4);
     put(o_ql, ql.data(), ql.size() * 8);
+    put(o_segb, seg_begin.data(), seg_begin.size() * 4);
+    put(o_csb, cs_begin.data(), cs_begin.size() * 4);
+    put(o_cs, cs.data(), cs.size() * 4);
+    const uint32_t n_type1 = (uint32_t)type1.size();
+    put(o_evc, &n_type1, 4);
     CU(ctx->d_batch_blob.reserve(blob.size(), 0, false, st));
     CU(cudaMemcpyAsync(ctx->d_batch_blob.p, blob.data(), blob.size(), cudaMemcpyHostToDevice, st));
     const size_t hist_words = (size_t)batch_hist_bins(n_len) * kBatchBin;
@@ -2848,9 +2898,17 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
     B.accum_len = ctx->d_batch_acc.as<unsigned long long>();
     B.accum_cand = reinterpret_cast<long long*>(B.accum_len + ((size_t)n_len + 1) * kAccumStride);
     B.hist = B.accum_len + ((size_t)n_len + 1) * kAccumStride + (size_t)n_cand * 4;
+    if (cov) {
+      CU(rs.d_ev.reserve((size_t)ev_cap * 8, 0, false, st));
+      if (n_type1) CU(cudaMemcpyAsync(rs.d_ev.p, type1.data(), (size_t)n_type1 * 8, cudaMemcpyHostToDevice, st));
+      B.seg_begin = reinterpret_cast<const int32_t*>(db + o_segb);
+      P.ev_keys = rs.d_ev.as<unsigned long long>();
+      P.ev_count = reinterpret_cast<uint32_t*>(db + o_evc);
+      P.ev_cap = (uint32_t)ev_cap;
+    }
     CU(cudaEventRecord(ctx->ev[1], st));
     launch_batch(P, B, (uint32_t)touch_total, ctx->d_batch_out.as<double>(),
-                 reinterpret_cast<const uint32_t*>(ctx->d_flags.as<unsigned long long>() + 1), ctx->sm_count, st);
+                 reinterpret_cast<const uint32_t*>(ctx->d_flags.as<unsigned long long>() + 1), ctx->sm_count, st, cov);
     CU(cudaEventRecord(ctx->ev[2], st));
     CU(cudaGetLastError());
     ctx->stats.kernel_launches += batch_launches(n_len, touch_total > 0);
@@ -2861,6 +2919,8 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
       ctx->stats.kernel_launches++;
     }
     CU(cudaMemcpyAsync(ctx->h_batch_out.data(), ctx->d_batch_out.p, (size_t)n_cand * kOutStride * 8, cudaMemcpyDeviceToHost, st));
+    uint32_t n_ev = 0;
+    if (cov) CU(cudaMemcpyAsync(&n_ev, db + o_evc, 4, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     {
       float ms = 0;
@@ -2870,7 +2930,40 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
     for (int c = 0; c < n_cand; c++) {
       const double* o = ctx->h_batch_out.data() + (size_t)c * kOutStride;
       if (((uint64_t)o[5]) & 2) return fail(ctx, GAML_ERR_CAPACITY, "placement scratch exhausted (GAML_B200_SCRATCH_ENTRIES)");
+      if (((uint64_t)o[5]) & 4) return fail(ctx, GAML_ERR_CAPACITY, "coverage-event buffer exhausted");
       for (int k = 0; k < GAML_PARTIAL_DOUBLES; k++) partials[((size_t)c * n_sets + s) * GAML_PARTIAL_DOUBLES + k] = o[k];
+    }
+    if (bad_bases)
+      for (int c = 0; c < n_cand; c++) bad_bases[(size_t)c * n_sets + s] = rs.bad_bases;
+    if (!cov) continue;
+    // the sweep over all segments: sort the emitted keys on the bits that can differ (33 below the segment id), one
+    // thread per event; bad[seg] = the segment's walk's bad bases over the current cache
+    int end_bit = 33;
+    while (end_bit < 64 && (1ull << (end_bit - 33)) < n_seg) end_bit++;
+    CU(rs.d_ev_sorted.reserve(std::max<size_t>(n_ev, 1) * 8, 0, false, st));
+    CU(rs.d_ev_temp.reserve(std::max<size_t>(coverage_sort_temp_bytes(n_ev, end_bit), 256), 0, false, st));
+    CU(rs.d_bad.reserve(std::max<size_t>(n_seg, 1) * 4, 0, false, st));
+    CU(cudaEventRecord(ctx->ev[1], st));
+    CU(cudaMemsetAsync(rs.d_bad.p, 0, std::max<size_t>(n_seg, 1) * 4, st));
+    CU(launch_coverage(rs.d_ev.as<unsigned long long>(), rs.d_ev_sorted.as<unsigned long long>(), n_ev, rs.d_ev_temp.p,
+                       rs.d_ev_temp.cap, reinterpret_cast<const int*>(db + o_csb), reinterpret_cast<const int*>(db + o_cs),
+                       rs.cfg.step, rs.cfg.insert_mean + 5 * rs.cfg.insert_std, rs.d_bad.as<int>(), ctx->sm_count, st, end_bit));
+    CU(cudaEventRecord(ctx->ev[2], st));
+    ctx->stats.kernel_launches += coverage_launches(end_bit);
+    std::vector<int32_t> bad(std::max<size_t>(n_seg, 1), 0);
+    CU(cudaMemcpyAsync(bad.data(), rs.d_bad.p, n_seg * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    {
+      float ms = 0;
+      if (cudaEventElapsedTime(&ms, ctx->ev[1], ctx->ev[2]) == cudaSuccess) batch_device_ms += ms;
+    }
+    ctx->stats.last_batch_cov_events += (int64_t)n_ev;
+    ctx->stats.last_batch_cov_segments += (int64_t)n_seg;
+    for (int c = 0; c < n_cand; c++) {   // bad_bases += added - erased, int arithmetic like the reference
+      int bb = rs.bad_bases;
+      const int n_erased = (int)cand_erased[c].size(), n_walks = n_erased + (int)cand_added[c].size();
+      for (int k = 0; k < n_walks; k++) bb += k < n_erased ? -bad[(size_t)seg_begin[c] + k] : bad[(size_t)seg_begin[c] + k];
+      bad_bases[(size_t)c * n_sets + s] = bb;
     }
   }
   // (measurement: the batch kernels' device time, and the whole call's wall time, in the fields of a normal evaluation)
@@ -3807,16 +3900,17 @@ int gaml_calc_prob_batch(gaml_ctx* ctx, int32_t n_cand, const int32_t* erased_id
   for (auto& rs : ctx->sets)
     if (rs->lo != 0 || rs->hi != rs->n_total)
       return fail(ctx, GAML_ERR_STATE, "gaml_calc_prob_batch on a sharded context: use gaml_calc_prob_batch_partial + gaml_combine_partials");
+  cudaSetDevice(ctx->device);
   const size_t n_sets = ctx->sets.size();
   std::vector<double> partials((size_t)n_cand * std::max<size_t>(n_sets, 1) * GAML_PARTIAL_DOUBLES);
-  std::vector<int32_t> tls(n_cand);
-  int rc = gaml_calc_prob_batch_partial(ctx, n_cand, erased_idx, erased_off, added_nodes, added_walk_off, cand_added_off,
-                                        partials.data(), tls.data());
+  std::vector<int32_t> tls(n_cand), bad((size_t)n_cand * std::max<size_t>(n_sets, 1));
+  int rc = calc_prob_batch_partial(ctx, n_cand, erased_idx, erased_off, added_nodes, added_walk_off, cand_added_off,
+                                   partials.data(), tls.data(), false, bad.data());
   if (rc) return rc;
   for (int c = 0; c < n_cand; c++) {
     gaml_result res;
     rc = combine(ctx, partials.data() + (size_t)c * n_sets * GAML_PARTIAL_DOUBLES, 1, tls[c], &res,
-                 zeros ? zeros + (size_t)c * 2 * n_sets : nullptr);
+                 zeros ? zeros + (size_t)c * 2 * n_sets : nullptr, bad.data() + (size_t)c * n_sets);
     if (rc) return rc;
     probs[c] = res.prob;
     if (total_lens) total_lens[c] = tls[c];

@@ -599,18 +599,32 @@ __device__ __forceinline__ unsigned order_few(Few& t) {
   return valid;
 }
 
+// A walk ordinal decides subtract (erased walk) versus add; it also names the walk a coverage event belongs to. An
+// evaluation passes its n_erased as a plain int (events under the ordinal); a penalised candidate batch passes CandWalks,
+// whose events go to the batch-global coverage segment seg_base + ordinal while the split stays candidate-local.
+struct CandWalks {
+  int n_erased;
+  int seg_base;
+};
+__device__ __forceinline__ bool is_erased(int walk, int n_erased) { return walk < n_erased; }
+__device__ __forceinline__ bool is_erased(int walk, const CandWalks& cw) { return walk < cw.n_erased; }
+__device__ __forceinline__ int event_walk(int walk, int) { return walk; }
+__device__ __forceinline__ int event_walk(int walk, const CandWalks& cw) { return cw.seg_base + walk; }
+
+template <class NE>
 __device__ __forceinline__ void one_pair(const ScoreParams& P, int xw, int xp, int xe, int yw, int yp, int ye, int l1,
-                                         int l2, double p1, double& acc, int n_erased) {
+                                         int l2, double p1, double& acc, NE n_erased) {
   if (xw != yw) return;
   double t;
-  if (pair_term(P, xw, xp, xe, yp, ye, l1, l2, p1, t)) acc = (xw < n_erased) ? __dsub_rn(acc, t) : __dadd_rn(acc, t);
+  if (pair_term(P, event_walk(xw, n_erased), xp, xe, yp, ye, l1, l2, p1, t))
+    acc = is_erased(xw, n_erased) ? __dsub_rn(acc, t) : __dadd_rn(acc, t);
 }
 
 // Per-read paired update for reads with <= kFew live placements per mate. For lists sorted in enumeration
 // order the plain x-major / y-minor loop with a same-walk filter IS the reference's order: walks ascend with
 // x, erased walks (subtract) precede added ones (add). Returns false if the read needs the scratch path.
-template <bool kCompact = false, class E0 = uint32_t, class E1 = uint32_t>
-__device__ __forceinline__ bool paired_read_with(const ScoreParams& P, const E0& lk0, const E1& lk1, int r, double& acc, int n_erased) {
+template <bool kCompact = false, class E0 = uint32_t, class E1 = uint32_t, class NE = int>
+__device__ __forceinline__ bool paired_read_with(const ScoreParams& P, const E0& lk0, const E1& lk1, int r, double& acc, NE n_erased) {
   Few a, b;
   const uint32_t ll = __ldg((kCompact ? P.clens : P.lens) + r);   // r is the list index k in the compact variant
   scan_two<kCompact>(P.m[0], lk0, r, a);
@@ -754,7 +768,8 @@ __device__ int gather_short(const MateView& mv, const E& epoch, int r, Plc* out)
   return n;
 }
 
-__device__ double apply_pairs(const ScoreParams& P, Plc* a, int n1, Plc* b, int n2, int l1, int l2, double acc, int n_erased) {
+template <class NE>
+__device__ double apply_pairs(const ScoreParams& P, Plc* a, int n1, Plc* b, int n2, int l1, int l2, double acc, NE n_erased) {
   sort_by_ord(a, n1);
   sort_by_ord(b, n2);
   // per-walk de-dup (lists are walk-major after the sort)
@@ -2182,11 +2197,19 @@ __global__ void __launch_bounds__(kBatchMaxLen) batch_prefix_kernel(const BatchP
 // fast read has only the one. The candidate's sums are reduced in the block and stored, no global atomics.
 constexpr int kCandKeys = 192;     // keys per mate staged in shared memory (more: looked up in global memory)
 constexpr int kCandRanges = 256;
+// Walk split of a candidate: its n_erased, and with kCov its first coverage segment (events of a penalised set).
+template <bool kCov>
+__device__ __forceinline__ auto cand_walks(const BatchParams& B, int c, int n_erased) {
+  if constexpr (kCov) return CandWalks{n_erased, __ldg(B.seg_begin + c)};
+  else return n_erased;
+}
+template <bool kCov>
 __global__ void __launch_bounds__(kBlock) batch_touch_kernel(const ScoreParams P, const BatchParams B) {
   if ((int)blockIdx.x >= B.n_blocks) return;
   const Int2 blk = B.blocks[blockIdx.x];   // {candidate, first record of this block's slice}
   const int c = blk.x;
   const BatchCand cd = B.cands[c];
+  const auto split = cand_walks<kCov>(B, c, cd.n_erased);
   const double2* log_tab = static_cast<const double2*>(P.log_tab);
   __shared__ int s_keys[2][kCandKeys];
   __shared__ int4 s_a[2][kCandKeys], s_b[2][kCandKeys];
@@ -2304,6 +2327,13 @@ __global__ void __launch_bounds__(kBlock) batch_touch_kernel(const ScoreParams P
               if (wrap_add(pos1, o1.z) >= o1.w && wrap_add(pos2, o2.z) >= o2.w) v1 = o1.x < cd.n_erased ? __dsub_rn(v1, t) : __dadd_rn(v1, t);
               if (b1.y == 2 && wrap_add(pos1, q1.z) >= q1.w && wrap_add(pos2, q2.z) >= q2.w)
                 v1 = q1.x < cd.n_erased ? __dsub_rn(v1, t) : __dadd_rn(v1, t);
+              if constexpr (kCov) {   // the coverage events of the same pair terms (emit_cov in pair_term, general replay)
+                const int l2 = (int)(__ldg(P.lens + r) >> 16);
+                if (wrap_add(pos1, o1.z) >= o1.w && wrap_add(pos2, o2.z) >= o2.w)
+                  emit_cov(P, event_walk(o1.x, split), wrap_add(pos1, o1.z), wrap_add(pos2, o2.z), l2, t);
+                if (b1.y == 2 && wrap_add(pos1, q1.z) >= q1.w && wrap_add(pos2, q2.z) >= q2.w)
+                  emit_cov(P, event_walk(q1.x, split), wrap_add(pos1, q1.z), wrap_add(pos2, q2.z), l2, t);
+              }
               account(r, v0, v1);
               done = true;
             }
@@ -2335,7 +2365,7 @@ __global__ void __launch_bounds__(kBlock) batch_touch_kernel(const ScoreParams P
       }
       const double v0 = P.values[r];
       double v1 = v0;
-      if (!paired_read_with(P, lk0, lk1, r, v1, cd.n_erased)) {
+      if (!paired_read_with(P, lk0, lk1, r, v1, split)) {
         // many-placement read: same replay from a scratch allocation, inline (rare)
         const int n1 = gather_short(P.m[0], lk0, r, nullptr), n2 = gather_short(P.m[1], lk1, r, nullptr);
         const unsigned long long at = atomicAdd(P.scratch_cursor, (unsigned long long)(n1 + n2));
@@ -2348,7 +2378,7 @@ __global__ void __launch_bounds__(kBlock) batch_touch_kernel(const ScoreParams P
         gather_short(P.m[0], lk0, r, a);
         gather_short(P.m[1], lk1, r, b);
         const uint32_t ll = __ldg(P.lens + r);
-        v1 = apply_pairs(P, a, n1, b, n2, ll & 0xffff, ll >> 16, v0, cd.n_erased);
+        v1 = apply_pairs(P, a, n1, b, n2, ll & 0xffff, ll >> 16, v0, split);
       }
       account(r, v0, v1);
     }
@@ -3223,7 +3253,7 @@ cudaError_t compact_copy(const uint32_t* list, int n_complex, const uint32_t* ro
 }
 
 void launch_batch(const ScoreParams& P, const BatchParams& B, uint32_t n_touch_records, double* out, const uint32_t* error_flag,
-                  int sm_count, cudaStream_t st) {
+                  int sm_count, cudaStream_t st, bool cov) {
   // GAML_B200_BATCH_TIMING=1 (measurement aid): per-kernel device times of the batch on stderr
   static const bool timing = getenv("GAML_B200_BATCH_TIMING") != nullptr;
   cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -3244,7 +3274,10 @@ void launch_batch(const ScoreParams& P, const BatchParams& B, uint32_t n_touch_r
     batch_prefix_kernel<<<1, kBatchMaxLen, 0, st>>>(B, j0, nb, (size_t)chunk * (kBatchMaxLen + 1));
   }
   if (timing) cudaEventRecord(ev[2], st);
-  if (n_touch_records > 0 && B.n_blocks > 0) batch_touch_kernel<<<B.n_blocks, kBlock, 0, st>>>(P, B);   // a block per slice of a candidate's records
+  if (n_touch_records > 0 && B.n_blocks > 0) {   // a block per slice of a candidate's records
+    if (cov) batch_touch_kernel<true><<<B.n_blocks, kBlock, 0, st>>>(P, B);
+    else batch_touch_kernel<false><<<B.n_blocks, kBlock, 0, st>>>(P, B);
+  }
   if (timing) cudaEventRecord(ev[3], st);
   batch_finalize_kernel<<<(B.n_cand + 127) / 128, 128, 0, st>>>(B, out, error_flag, (long long)P.n_reads);
   if (timing) {
@@ -3485,17 +3518,21 @@ void launch_cdesc_fill(const uint32_t* list, int n_complex, const uint32_t* lens
     cdesc_fill_kernel<<<(n_complex + 255) / 256, 256, 0, st>>>(list, n_complex, lens, cptr1, cptr2, static_cast<int4*>(desc));
 }
 
-size_t coverage_sort_temp_bytes(unsigned n) {
+size_t coverage_sort_temp_bytes(unsigned n, int end_bit) {
   size_t need = 0;
-  cub::DeviceRadixSort::SortKeys(nullptr, need, (const unsigned long long*)nullptr, (unsigned long long*)nullptr, (int)n);
+  cub::DeviceRadixSort::SortKeys(nullptr, need, (const unsigned long long*)nullptr, (unsigned long long*)nullptr, (int)n, 0, end_bit);
   return need;
+}
+
+int coverage_launches(int end_bit) {
+  return 2 + (end_bit + 7) / 8 + 1;   // CUB onesweep: histogram + scan + one pass per 8-bit digit; then the sweep
 }
 
 cudaError_t launch_coverage(const unsigned long long* keys_in, unsigned long long* keys_sorted, unsigned n, void* temp,
                             size_t temp_bytes, const int* cs_begin, const int* cs, double step, double min_from_start, int* bad,
-                            int sm_count, cudaStream_t st) {
+                            int sm_count, cudaStream_t st, int end_bit) {
   size_t need = temp_bytes;
-  cudaError_t err = cub::DeviceRadixSort::SortKeys(temp, need, keys_in, keys_sorted, (int)n, 0, 64, st);
+  cudaError_t err = cub::DeviceRadixSort::SortKeys(temp, need, keys_in, keys_sorted, (int)n, 0, end_bit, st);
   if (err != cudaSuccess) return err;
   coverage_sweep_kernel<<<grid_for(n, 256, sm_count, 8), 256, 0, st>>>(keys_sorted, n, cs_begin, cs, step, min_from_start, bad);
   return cudaGetLastError();

@@ -77,8 +77,9 @@ cudaError_t compact_offsets(const uint32_t* list, int n_complex, const uint32_t*
 cudaError_t compact_copy(const uint32_t* list, int n_complex, const uint32_t* rowptr, const uint32_t* cptr, const void* rows,
                          void* crows, cudaStream_t st, int* launches);
 // Batched candidate evaluation of one paired set: base pass per distinct total length, touched-read pass, finalize.
+// cov: the touched-read pass also emits the coverage events of every pair term (P.ev_keys, under B.seg_begin segments).
 void launch_batch(const ScoreParams& P, const BatchParams& B, uint32_t n_touch_records, double* out, const uint32_t* error_flag,
-                  int sm_count, cudaStream_t st);
+                  int sm_count, cudaStream_t st, bool cov = false);
 int batch_hist_bins(int n_len);            // bins of BatchParams::hist for n_len distinct total lengths
 int batch_launches(int n_len, bool touch);  // kernels launch_batch issues
 // Term table of a uniform-length paired set: 1 + (1 << shift)^2 * ins_n TermEntry (entry 0 = "no pair term").
@@ -111,11 +112,13 @@ size_t perm_temp_bytes(int n);
 cudaError_t build_read_permutation(const void* fast, int n, unsigned long long* keys, uint32_t* ids, uint32_t* inv, uint32_t* n_fast,
                                    void* temp, size_t temp_bytes, cudaStream_t st, int* launches);
 void launch_remap_arena(void* arena, size_t n_records, const uint32_t* inv, int sm_count, cudaStream_t st);
-// Coverage-gap penalty of one paired set: radix sort of the event keys, then the one-thread-per-event sweep.
-size_t coverage_sort_temp_bytes(unsigned n);
+// Coverage-gap penalty of one paired set: radix sort of the event keys, then the one-thread-per-event sweep. The sort
+// looks at key bits [0, end_bit): 33 position / type bits below the walk id, so fewer when the walk ids are few.
+size_t coverage_sort_temp_bytes(unsigned n, int end_bit = 64);
 cudaError_t launch_coverage(const unsigned long long* keys_in, unsigned long long* keys_sorted, unsigned n, void* temp,
                             size_t temp_bytes, const int* cs_begin, const int* cs, double step, double min_from_start, int* bad,
-                            int sm_count, cudaStream_t st);
+                            int sm_count, cudaStream_t st, int end_bit = 64);
+int coverage_launches(int end_bit);   // kernels launch_coverage issues for a sort large enough for CUB's onesweep path
 // PacBio coverage penalty of one set: emit intervals, sort by (walk, start), running max of ends, sort positions, sweep.
 size_t pacbio_coverage_temp_bytes(uint32_t cap);
 cudaError_t launch_pacbio_coverage(const PbCovParams& C, unsigned long long* packed, unsigned long long* run_max, void* temp,

@@ -26,7 +26,7 @@ enum {
   GAML_ERR_CUDA = -1,          /* CUDA runtime / no device */
   GAML_ERR_ARG = -2,           /* bad argument */
   GAML_ERR_KEY_EXISTS = -3,    /* cache key inserted twice */
-  GAML_ERR_UNSUPPORTED = -4,   /* e.g. a penalised paired / PacBio set on a read-id shard, a batch over non-paired sets */
+  GAML_ERR_UNSUPPORTED = -4,   /* e.g. a batch over non-paired sets, or a penalised set in a _partial / _gathered batch */
   GAML_ERR_CAPACITY = -5,      /* a read needs more placement scratch than configured */
   GAML_ERR_STATE = -6          /* call order (e.g. finalize without a pending evaluation) */
 };
@@ -110,6 +110,9 @@ typedef struct {
   int64_t full_reuse_evals;        /* full evaluations of the walk list evaluated last: slot tables already on the device, no upload */
   int64_t full_patch_evals;        /* full evaluations of a list a few walks away from the resident one: only the slot updates of
                                       those walks' keys were built and uploaded (O(changed walks) host work) */
+  int64_t last_batch_cov_events;   /* coverage-gap events (contig starts + covered positions) the last candidate batch sorted and
+                                      swept, over its penalised paired sets; 0 without such a set */
+  int64_t last_batch_cov_segments; /* coverage segments of that batch: one per (candidate, erased or added walk, penalised set) */
 } gaml_stats;
 
 /* ---- context ---------------------------------------------------------------------------- */
@@ -242,8 +245,12 @@ int gaml_calc_prob_gathered(gaml_ctx* ctx, const int32_t* walk_nodes, const int6
  * layout of gaml_calc_prob). probs[c] is exactly the double gaml_calc_prob would return for that walk set if it were
  * called now — the same per-read subtract/add replay from the current ScoringState and the same exact sum — but
  * nothing is committed, so a move (LocalChange2, FixRepForNode2, FixGapLength: moves.cc:107-113, 715-726, 1158-1203)
- * can score all its candidates in one launch and then commit the winner with gaml_calc_prob. Paired sets only.
- * zeros (optional): n_cand x 2 n_sets. The _partial form returns n_cand x n_sets x GAML_PARTIAL_DOUBLES for shards. */
+ * can score all its candidates in one launch and then commit the winner with gaml_calc_prob. Paired sets only. A set
+ * with penalty_constant != 0 is scored with the candidate's own bad bases (the state's, minus the erased walks', plus the
+ * added walks', each swept over the current cache: graph.cc:1938, 1946, 1988) on an unsharded context.
+ * zeros (optional): n_cand x 2 n_sets. The _partial form returns n_cand x n_sets x GAML_PARTIAL_DOUBLES for shards; it
+ * refuses a penalised set (GAML_ERR_UNSUPPORTED): partials carry no bad bases, gaml_combine_partials would apply the
+ * base state's. */
 int gaml_calc_prob_batch(gaml_ctx* ctx, int32_t n_cand, const int32_t* erased_idx, const int64_t* erased_off,
                          const int32_t* added_nodes, const int64_t* added_walk_off, const int64_t* cand_added_off,
                          double* probs, int32_t* total_lens, int32_t* zeros);
@@ -253,7 +260,8 @@ int gaml_calc_prob_batch_partial(gaml_ctx* ctx, int32_t n_cand, const int32_t* e
 
 /* The multi-GPU form (read-id shards, one context per GPU, every rank calls it with the same candidates): the shards'
  * partials of all candidates are summed by ONE all-reduce on the library's stream (needs gaml_nccl_exchange_init) and
- * combined exactly, so every rank receives the same probs — bit-identical to the unsharded gaml_calc_prob_batch. */
+ * combined exactly, so every rank receives the same probs — bit-identical to the unsharded gaml_calc_prob_batch.
+ * A penalised set is refused (GAML_ERR_UNSUPPORTED): every candidate's coverage events would have to be all-gathered. */
 int gaml_calc_prob_batch_gathered(gaml_ctx* ctx, int32_t n_cand, const int32_t* erased_idx, const int64_t* erased_off,
                                   const int32_t* added_nodes, const int64_t* added_walk_off, const int64_t* cand_added_off,
                                   double* probs, int32_t* total_lens, int32_t* zeros);

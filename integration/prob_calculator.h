@@ -101,7 +101,8 @@ class ProbCalculator {
   // in one device batch (gaml_calc_prob_batch) and changes no state. scores[c] is the double a CalcProb(candidates[c])
   // issued right now would return. The moves that try several alternatives one CalcProb at a time (LocalChange2
   // moves.cc:107-113, FixGapLength 715-726, FixRepForNode2 1158-1305) submit them here when built with
-  // oracle/build_ref.sh's moves.cc patch (target gaml_gpu_batched, GamlBatchReplay below). With single or PacBio sets
+  // oracle/build_ref.sh's moves.cc patch (target gaml_gpu_batched, GamlBatchReplay below). Paired sets with a
+  // coverage-gap penalty are batched too (each candidate gets its own bad bases). With single or PacBio sets
   // configured — they keep no incremental state to evaluate candidates against — the candidates are scored one by one.
   vector<double> CalcProbBatch(vector<vector<vector<int>>>& candidates) {
     vector<double> scores(candidates.size(), 0.0);

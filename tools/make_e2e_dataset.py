@@ -29,6 +29,10 @@ def main():
     ap.add_argument("--n-reads", type=int, default=50000)
     ap.add_argument("--iterations", type=int, default=500)
     ap.add_argument("--seed", type=int, default=7)
+    # coverage-gap penalty of the paired set (PrepareReadSetFromConfig, gaml.cc:783-872: the paired sweep's step is
+    # insert_mean - penalty_step); both omitted: no penalty keys, the reference's defaults
+    ap.add_argument("--penalty-constant", type=float, default=None)
+    ap.add_argument("--penalty-step", type=float, default=None)
     args = ap.parse_args()
     os.makedirs(args.outdir, exist_ok=True)
     rng = np.random.default_rng(args.seed)
@@ -91,6 +95,10 @@ def main():
         fastq(os.path.join(args.outdir, "reads_2.fastq"), r2)
         cfg += ["[rs]", "type=paired", f"filename1={args.outdir}/reads_1.fastq", f"filename2={args.outdir}/reads_2.fastq",
                 "insert_mean=300", "insert_std=30", f"cache_prefix={args.outdir}/nocache"]
+        if args.penalty_constant is not None:
+            cfg.append(f"penalty_constant={args.penalty_constant:g}")
+        if args.penalty_step is not None:
+            cfg.append(f"penalty_step={args.penalty_step:g}")
     with open(os.path.join(args.outdir, "gaml.cfg"), "w") as f:
         f.write("\n".join(cfg) + "\n")
     print(f"genome {len(genome)} bp, {len(nodes)} nodes, {args.n_reads} {args.kind} reads -> {args.outdir}")

@@ -9,12 +9,17 @@ ITERS=${2:-500}
 KINDS=${E2E_KINDS:-"single paired"}     # E2E_KINDS=paired E2E_UNIQUE=100 E2E_READS=400000: a 1 Mbp / 400 k-pair run
 UNIQUE=${E2E_UNIQUE:-10}
 READS=${E2E_READS:-50000}
+PENALTY=()                               # E2E_PENALTY="<penalty_constant> <penalty_step>": the paired set's coverage-gap penalty
+if [ -n "${E2E_PENALTY:-}" ]; then
+  read -r pc ps <<< "$E2E_PENALTY"
+  PENALTY=(--penalty-constant "$pc" --penalty-step "$ps")
+fi
 mkdir -p "$OUT"
 rc=0
 for kind in $KINDS; do
   D=/tmp/e2e_$kind
   rm -rf "$D"
-  python "$ROOT/tools/make_e2e_dataset.py" "$D" --kind $kind --n-unique "$UNIQUE" --n-reads "$READS" --iterations "$ITERS" > "$OUT/$kind.gen.log"
+  python "$ROOT/tools/make_e2e_dataset.py" "$D" --kind $kind --n-unique "$UNIQUE" --n-reads "$READS" --iterations "$ITERS" "${PENALTY[@]}" > "$OUT/$kind.gen.log"
   t0=$(date +%s.%N)
   ( cd "$D" && stdbuf -oL "$ROOT/oracle/_ref/gaml_ref" gaml.cfg > ref.log 2>&1 )
   t1=$(date +%s.%N)
