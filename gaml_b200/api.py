@@ -48,7 +48,8 @@ class Stats(C.Structure):
                 ("last_scratch_placements", C.c_int64), ("last_multi_items", C.c_int64),
                 ("fast_change_evals", C.c_int64), ("delta_only_evals", C.c_int64), ("cache_appends", C.c_int64),
                 ("cache_rebuilds", C.c_int64), ("full_reuse_evals", C.c_int64), ("full_patch_evals", C.c_int64),
-                ("last_batch_cov_events", C.c_int64), ("last_batch_cov_segments", C.c_int64)]
+                ("last_batch_cov_events", C.c_int64), ("last_batch_cov_segments", C.c_int64),
+                ("last_batch_cov_exported", C.c_int64)]
 
 
 EXPORTS = ["gaml_ctx_create", "gaml_ctx_destroy", "gaml_last_error", "gaml_ctx_stream", "gaml_set_graph",
@@ -60,7 +61,8 @@ EXPORTS = ["gaml_ctx_create", "gaml_ctx_destroy", "gaml_last_error", "gaml_ctx_s
            "gaml_eval_finish_gathered", "gaml_calc_prob_gathered", "gaml_cache_save", "gaml_cache_load",
            "gaml_pacbio_alignment_logprob", "gaml_peer_exchange_create", "gaml_peer_exchange_open", "gaml_peer_exchange_close",
            "gaml_nccl_unique_id", "gaml_nccl_exchange_init", "gaml_calc_prob_batch_gathered",
-           "gaml_penalty_export", "gaml_penalty_import"]
+           "gaml_penalty_export", "gaml_penalty_import", "gaml_calc_prob_batch_shard", "gaml_batch_penalty_export",
+           "gaml_batch_penalty_import", "gaml_combine_batch_partials"]
 
 _lib = None
 
@@ -114,6 +116,10 @@ def load_library() -> C.CDLL:
     lib.gaml_calc_prob_batch_gathered.argtypes = [vp, C.c_int32, i32p, i64p, i32p, i64p, i64p, dp, i32p, i32p]
     lib.gaml_penalty_export.argtypes = [vp, C.c_int, C.POINTER(C.c_uint64), C.c_int64, C.POINTER(C.c_int64)]
     lib.gaml_penalty_import.argtypes = [vp, C.c_int, C.POINTER(C.c_uint64), C.c_int64]
+    lib.gaml_calc_prob_batch_shard.argtypes = [vp, C.c_int32, i32p, i64p, i32p, i64p, i64p, dp, i32p]
+    lib.gaml_batch_penalty_export.argtypes = [vp, C.c_int, C.POINTER(C.c_uint64), C.c_int64, C.POINTER(C.c_int64)]
+    lib.gaml_batch_penalty_import.argtypes = [vp, C.c_int, C.POINTER(C.c_uint64), C.c_int64]
+    lib.gaml_combine_batch_partials.argtypes = [vp, dp, C.c_int32, C.c_int32, dp, i32p]
     lib.gaml_peer_exchange_create.argtypes = [vp, C.c_int32, C.c_int32, vp, C.POINTER(vp)]
     lib.gaml_peer_exchange_open.argtypes = [vp, vp, C.POINTER(vp)]
     lib.gaml_peer_exchange_close.argtypes = [vp]
@@ -382,6 +388,47 @@ class ProbCalculator:
                                                            w_off.ctypes.data_as(i64p), ca_off.ctypes.data_as(i64p),
                                                            probs.ctypes.data_as(C.POINTER(C.c_double)), _p32(tls), _p32(zeros)))
         return probs, tls
+
+    def calc_prob_batch_shard_packed(self, packed):
+        """gaml_calc_prob_batch_shard: this shard's partials of every candidate (penalised sets included; their coverage waits
+        for batch_penalty_export / _import) -> (partials [n, sets, PARTIAL_DOUBLES], total_lens [n])."""
+        n, er_a, er_off, nodes, w_off, ca_off = packed
+        ns = max(len(self.sets), 1)
+        part = np.zeros(n * ns * PARTIAL_DOUBLES, dtype=np.float64)
+        tls = np.zeros(n, dtype=np.int32)
+        i64p = C.POINTER(C.c_int64)
+        self._check(self.lib.gaml_calc_prob_batch_shard(self.h, n, _p32(er_a), er_off.ctypes.data_as(i64p), _p32(nodes),
+                                                        w_off.ctypes.data_as(i64p), ca_off.ctypes.data_as(i64p),
+                                                        part.ctypes.data_as(C.POINTER(C.c_double)), _p32(tls)))
+        return part.reshape(n, ns, PARTIAL_DOUBLES), tls
+
+    def batch_penalty_export(self, set_id: int) -> np.ndarray:
+        """gaml_batch_penalty_export: this shard's thinned coverage keys of the pending shard batch (uint64)."""
+        n = C.c_int64(0)
+        rc = self.lib.gaml_batch_penalty_export(self.h, set_id, None, 0, C.byref(n))
+        if rc < 0 and n.value == 0:
+            self._check(rc)
+        out = np.zeros(max(n.value, 1), dtype=np.uint64)
+        self._check(self.lib.gaml_batch_penalty_export(self.h, set_id, out.ctypes.data_as(C.POINTER(C.c_uint64)), n.value,
+                                                       C.byref(n)))
+        return out[:n.value]
+
+    def batch_penalty_import(self, set_id: int, all_keys: np.ndarray) -> None:
+        """gaml_batch_penalty_import: the concatenation of every shard's exported keys (this shard's included)."""
+        a = np.ascontiguousarray(all_keys, dtype=np.uint64)
+        p = a.ctypes.data_as(C.POINTER(C.c_uint64)) if len(a) else None
+        self._check(self.lib.gaml_batch_penalty_import(self.h, set_id, p, len(a)))
+
+    def combine_batch_partials(self, gathered: np.ndarray):
+        """gaml_combine_batch_partials: gathered [n_shards, n, sets, PARTIAL_DOUBLES] -> (probs [n], zeros [n, sets, 2])."""
+        g = np.ascontiguousarray(gathered, dtype=np.float64)
+        ns = max(len(self.sets), 1)
+        n_shards, n = g.shape[0], g.shape[1]
+        probs = np.zeros(n, dtype=np.float64)
+        zeros = np.zeros(n * 2 * ns, dtype=np.int32)
+        self._check(self.lib.gaml_combine_batch_partials(self.h, g.ctypes.data_as(C.POINTER(C.c_double)), n_shards, n,
+                                                         probs.ctypes.data_as(C.POINTER(C.c_double)), _p32(zeros)))
+        return probs, zeros.reshape(n, ns, 2)
 
     def calc_prob_batch(self, candidates):
         """candidates: list of (erased base-walk indices, added walks). -> (probs [n], total_lens [n], zeros [n][sets]).

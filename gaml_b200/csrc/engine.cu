@@ -234,6 +234,19 @@ struct ReadSetState {
   bool penalty_pending = false;
   std::vector<unsigned long long> h_type1;   // the host's contig-start events of the pending evaluation (paired)
   DevBuf d_cov_thr, d_ev, d_ev_sorted, d_ev_temp, d_bad;
+  // a penalised set of a shard candidate batch (gaml_calc_prob_batch_shard) waiting for every shard's thinned coverage
+  // events (gaml_batch_penalty_export / _import); the batch's segment tables are kept for the import's sweep
+  struct {
+    bool pending = false, imported = false;
+    std::vector<int32_t> seg_begin;          // n_cand + 1: candidate c owns segments [seg_begin[c], seg_begin[c + 1])
+    std::vector<int32_t> n_erased;           // per candidate: its first n_erased segments are erased walks
+    std::vector<int32_t> cs_begin, cs;       // contig starts per segment
+    std::vector<unsigned long long> type1;   // their keys
+    int end_bit = 33;
+    uint32_t n_thin = 0;                     // this shard's kept keys, in d_thin
+    std::vector<int32_t> bad;                // after the import: every candidate's bad bases
+    DevBuf d_thin, d_state, d_cs;
+  } sb;
   // PacBio coverage penalty (graph.cc:3197-3250)
   bool pb_penalty = false;
   DevBuf d_pb_ikey, d_pb_iend, d_pb_pkey, d_pb_packed, d_pb_runmax, d_pb_temp, d_pb_count;
@@ -335,6 +348,10 @@ struct gaml_ctx {
   size_t h_blob_cap = 0;
   DevBuf d_flags, d_scratch, d_csr_temp, d_logtab;
   DevBuf d_batch_blob, d_batch_acc, d_batch_out;   // gaml_calc_prob_batch
+  // the pending shard candidate batch (gaml_calc_prob_batch_shard until gaml_combine_batch_partials; any later evaluation,
+  // batch or gaml_reset_state drops it): its candidate count and total lengths; the sets keep their coverage part (sb)
+  bool shard_batch = false;
+  std::vector<int32_t> shard_batch_lens;
   DevBuf d_aln[8];                                  // gaml_pacbio_alignment_logprob
   std::vector<double> h_batch_out;
   void* h_append_pinned = nullptr;                  // pinned staging of a cache append (arena records, rows, groups, lists, key-map patches)
@@ -427,6 +444,13 @@ namespace {
 int fail(gaml_ctx* ctx, int code, const std::string& msg) {
   ctx->error = msg;
   return code;
+}
+
+// A shard candidate batch is stateless, so dropping it is always safe; its coverage tables describe the base state it was
+// scored against, which the next evaluation, batch or reset replaces.
+void discard_shard_batch(gaml_ctx* ctx) {
+  ctx->shard_batch = false;
+  for (auto& rs : ctx->sets) rs->sb.pending = rs->sb.imported = false;
 }
 
 // d_flags layout (u64 words, zeroed at the start of every evaluation): [0] scratch cursor | [1] error flag (u32) |
@@ -1442,6 +1466,7 @@ int prepare(gaml_ctx* ctx, const int32_t* nodes, const int64_t* offs, int n_walk
   PrepTimer pt;
   if (n_walks < 0 || (n_walks > 0 && (!nodes || !offs))) return fail(ctx, GAML_ERR_ARG, "bad walk arrays");
   if (ctx->node_len.empty()) return fail(ctx, GAML_ERR_STATE, "gaml_set_graph has not been called");
+  discard_shard_batch(ctx);
   // an evaluation in flight updates the read state and the walk bookkeeping when it is finished: preparing another one
   // underneath it would score deltas against the wrong old walks
   if (ctx->launched) return fail(ctx, GAML_ERR_STATE, "an evaluation is in flight: call gaml_eval_finish before preparing the next one");
@@ -2606,9 +2631,13 @@ int combine(gaml_ctx* ctx, const double* gathered, int n_shards, int total_len, 
 // are scored only when it is given (unsharded contexts: gaml_calc_prob_batch), because the partials alone carry no bad
 // bases: bad_bases_c = the state's - sum over the erased walks + sum over the added walks of the walk's own sweep over the
 // current cache (EraseFromScoringState / AddToScoringState, graph.cc:1938, 1946), one coverage segment per such walk.
+// shard (gaml_calc_prob_batch_shard): a penalised set's events of this shard are sorted and thinned instead of swept, and
+// the batch stays pending until every shard's thinned events are imported (gaml_batch_penalty_import).
 int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx, const int64_t* erased_off,
                             const int32_t* added_nodes, const int64_t* added_walk_off, const int64_t* cand_added_off,
-                            double* partials, int32_t* total_lens, bool reduce_over_ranks = false, int32_t* bad_bases = nullptr) {
+                            double* partials, int32_t* total_lens, bool reduce_over_ranks = false, int32_t* bad_bases = nullptr,
+                            bool shard = false) {
+  discard_shard_batch(ctx);
   if (n_cand <= 0 || !erased_off || !cand_added_off || !added_walk_off || !partials)
     return fail(ctx, GAML_ERR_ARG, "bad batch arguments");
   const auto t_batch0 = std::chrono::steady_clock::now();
@@ -2624,7 +2653,7 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
     if (rs->penalty && reduce_over_ranks)
       return fail(ctx, GAML_ERR_UNSUPPORTED, "gaml_calc_prob_batch_gathered with penalty_constant != 0 is not supported: every "
                                              "candidate's coverage events would have to be all-gathered over the read-id shards");
-    if (rs->penalty && !bad_bases)
+    if (rs->penalty && !bad_bases && !shard)
       return fail(ctx, GAML_ERR_UNSUPPORTED, "gaml_calc_prob_batch_partial with penalty_constant != 0 is not supported: the partials "
                                              "carry no bad bases, so gaml_combine_partials would apply the base state's value "
                                              "(use gaml_calc_prob_batch)");
@@ -2713,7 +2742,7 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
   for (size_t j = 0; j < two_lens.size(); j++) ql[j] = fix_log_host((double)two_lens[j]);
   const int n_len = (int)two_lens.size();
   ctx->h_batch_out.assign((size_t)n_cand * kOutStride, 0.0);
-  ctx->stats.last_batch_cov_events = ctx->stats.last_batch_cov_segments = 0;
+  ctx->stats.last_batch_cov_events = ctx->stats.last_batch_cov_segments = ctx->stats.last_batch_cov_exported = 0;
   cudaStream_t st = ctx->stream;
 
   for (size_t s = 0; s < n_sets; s++) {
@@ -2940,6 +2969,42 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
     // thread per event; bad[seg] = the segment's walk's bad bases over the current cache
     int end_bit = 33;
     while (end_bit < 64 && (1ull << (end_bit - 33)) < n_seg) end_bit++;
+    if (shard) {
+      // this shard's covered positions only (the type-1 keys lead the buffer and stay on the host): sort, thin, keep
+      auto& sb = rs.sb;
+      const uint32_t n_emit = n_ev - n_type1;
+      CU(rs.d_ev_sorted.reserve(std::max<size_t>(n_emit, 1) * 8, 0, false, st));
+      CU(rs.d_ev_temp.reserve(std::max<size_t>(coverage_sort_temp_bytes(n_emit, end_bit), 256), 0, false, st));
+      CU(sb.d_thin.reserve(std::max<size_t>(n_emit, 1) * 8, 0, false, st));
+      CU(sb.d_state.reserve(coverage_thin_state_bytes(n_emit), 0, false, st));
+      CU(cudaEventRecord(ctx->ev[1], st));
+      CU(launch_coverage_thin(rs.d_ev.as<unsigned long long>() + n_type1, rs.d_ev_sorted.as<unsigned long long>(), n_emit,
+                              rs.d_ev_temp.p, rs.d_ev_temp.cap, end_bit, rs.cfg.step, sb.d_thin.as<unsigned long long>(),
+                              sb.d_state.as<unsigned long long>(), st));
+      CU(cudaEventRecord(ctx->ev[2], st));
+      if (n_emit) ctx->stats.kernel_launches += coverage_launches(end_bit);
+      unsigned long long n_thin = 0;
+      CU(cudaMemcpyAsync(&n_thin, sb.d_state.as<unsigned long long>() + 1, 8, cudaMemcpyDeviceToHost, st));
+      CU(cudaStreamSynchronize(st));
+      {
+        float ms = 0;
+        if (cudaEventElapsedTime(&ms, ctx->ev[1], ctx->ev[2]) == cudaSuccess) batch_device_ms += ms;
+      }
+      sb.seg_begin = seg_begin;
+      sb.seg_begin.push_back((int32_t)n_seg);
+      sb.n_erased.resize(n_cand);
+      for (int c = 0; c < n_cand; c++) sb.n_erased[c] = (int32_t)cand_erased[c].size();
+      sb.cs_begin = std::move(cs_begin);
+      sb.cs = std::move(cs);
+      sb.type1 = std::move(type1);
+      sb.end_bit = end_bit;
+      sb.n_thin = (uint32_t)n_thin;
+      sb.pending = true;
+      ctx->stats.last_batch_cov_events += (int64_t)n_ev;
+      ctx->stats.last_batch_cov_segments += (int64_t)n_seg;
+      ctx->stats.last_batch_cov_exported += (int64_t)n_thin;
+      continue;
+    }
     CU(rs.d_ev_sorted.reserve(std::max<size_t>(n_ev, 1) * 8, 0, false, st));
     CU(rs.d_ev_temp.reserve(std::max<size_t>(coverage_sort_temp_bytes(n_ev, end_bit), 256), 0, false, st));
     CU(rs.d_bad.reserve(std::max<size_t>(n_seg, 1) * 4, 0, false, st));
@@ -2966,6 +3031,10 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
       bad_bases[(size_t)c * n_sets + s] = bb;
     }
   }
+  if (shard) {
+    ctx->shard_batch = true;
+    ctx->shard_batch_lens = cand_len;
+  }
   // (measurement: the batch kernels' device time, and the whole call's wall time, in the fields of a normal evaluation)
   ctx->stats.last_device_ms = batch_device_ms;
   ctx->stats.last_prepare_host_us = std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t_batch0).count();
@@ -2974,6 +3043,15 @@ int calc_prob_batch_partial(gaml_ctx* ctx, int n_cand, const int32_t* erased_idx
 }
 
 int check_ctx(gaml_ctx* ctx) { return ctx ? GAML_OK : GAML_ERR_ARG; }
+
+// GAML_OK when the read set has a pending shard batch's coverage (a penalised set of gaml_calc_prob_batch_shard)
+int shard_batch_set(gaml_ctx* ctx, int set, const char* what) {
+  if (set < 0 || set >= (int)ctx->sets.size()) return fail(ctx, GAML_ERR_ARG, "no such read set");
+  if (!ctx->shard_batch || !ctx->sets[set]->sb.pending)
+    return fail(ctx, GAML_ERR_STATE, std::string(what) + ": no pending shard batch with a penalty on this read set (the set has "
+                                     "no penalty, or no gaml_calc_prob_batch_shard since the last evaluation, batch or reset)");
+  return GAML_OK;
+}
 
 }  // namespace
 }  // namespace gaml
@@ -3942,6 +4020,110 @@ int gaml_calc_prob_batch_gathered(gaml_ctx* ctx, int32_t n_cand, const int32_t* 
   return GAML_OK;
 }
 
+int gaml_calc_prob_batch_shard(gaml_ctx* ctx, int32_t n_cand, const int32_t* erased_idx, const int64_t* erased_off,
+                               const int32_t* added_nodes, const int64_t* added_walk_off, const int64_t* cand_added_off,
+                               double* partials, int32_t* total_lens) {
+  if (check_ctx(ctx)) return GAML_ERR_ARG;
+  for (auto& rs : ctx->sets)   // the candidates start from the state's bad bases, and the evaluation's events sit in d_ev
+    if (rs->penalty_pending)
+      return fail(ctx, GAML_ERR_STATE, "gaml_calc_prob_batch_shard while an evaluation's coverage events are pending: finish "
+                                       "the evaluation with gaml_penalty_export / gaml_penalty_import first");
+  cudaSetDevice(ctx->device);
+  return calc_prob_batch_partial(ctx, n_cand, erased_idx, erased_off, added_nodes, added_walk_off, cand_added_off, partials,
+                                 total_lens, false, nullptr, true);
+}
+
+int gaml_batch_penalty_export(gaml_ctx* ctx, int set, uint64_t* out, int64_t cap, int64_t* n_out) {
+  if (check_ctx(ctx) || !n_out) return GAML_ERR_ARG;
+  const int rc = shard_batch_set(ctx, set, "gaml_batch_penalty_export");
+  if (rc) return rc;
+  auto& sb = ctx->sets[set]->sb;
+  *n_out = sb.n_thin;
+  if ((int64_t)sb.n_thin > cap) return fail(ctx, GAML_ERR_CAPACITY, "gaml_batch_penalty_export: output buffer too small (n_out holds the count)");
+  if (sb.n_thin && !out) return fail(ctx, GAML_ERR_ARG, "gaml_batch_penalty_export: out is NULL");
+  cudaSetDevice(ctx->device);
+  if (sb.n_thin) CU(cudaMemcpyAsync(out, sb.d_thin.p, (size_t)sb.n_thin * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  return GAML_OK;
+}
+
+int gaml_batch_penalty_import(gaml_ctx* ctx, int set, const uint64_t* all, int64_t n_all) {
+  if (check_ctx(ctx) || n_all < 0 || (n_all > 0 && !all)) return GAML_ERR_ARG;
+  int rc = shard_batch_set(ctx, set, "gaml_batch_penalty_import");
+  if (rc) return rc;
+  ReadSetState& rs = *ctx->sets[set];
+  auto& sb = rs.sb;
+  const size_t n_seg = sb.cs_begin.size() - 1;
+  // [contig starts | every shard's kept keys] -> the same sort and sweep as the unsharded batch
+  const uint64_t total = (uint64_t)sb.type1.size() + (uint64_t)n_all;
+  if (total > 0x7fffffffull) return fail(ctx, GAML_ERR_CAPACITY, "too many coverage events");
+  for (int64_t i = 0; i < n_all; i++)   // the sweep indexes the segment tables with the key's segment
+    if ((all[i] >> 33) >= n_seg || !(all[i] & 1))
+      return fail(ctx, GAML_ERR_ARG, "gaml_batch_penalty_import: a key that no shard of this batch exported");
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = ctx->stream;
+  std::vector<unsigned long long> keys((size_t)std::max<uint64_t>(total, 1));
+  std::copy(sb.type1.begin(), sb.type1.end(), keys.begin());
+  if (n_all) memcpy(keys.data() + sb.type1.size(), all, (size_t)n_all * 8);
+  std::vector<int32_t> tables(sb.cs_begin);
+  tables.insert(tables.end(), sb.cs.begin(), sb.cs.end());
+  CU(rs.d_ev.reserve(keys.size() * 8, 0, false, st));
+  CU(rs.d_ev_sorted.reserve(keys.size() * 8, 0, false, st));
+  CU(rs.d_ev_temp.reserve(std::max<size_t>(coverage_sort_temp_bytes((unsigned)total, sb.end_bit), 256), 0, false, st));
+  CU(rs.d_bad.reserve(std::max<size_t>(n_seg, 1) * 4, 0, false, st));
+  CU(sb.d_cs.reserve(tables.size() * 4, 0, false, st));
+  CU(cudaMemcpyAsync(rs.d_ev.p, keys.data(), (size_t)total * 8, cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(sb.d_cs.p, tables.data(), tables.size() * 4, cudaMemcpyHostToDevice, st));
+  CU(cudaMemsetAsync(rs.d_bad.p, 0, std::max<size_t>(n_seg, 1) * 4, st));
+  const int* d_csb = sb.d_cs.as<int>();
+  CU(launch_coverage(rs.d_ev.as<unsigned long long>(), rs.d_ev_sorted.as<unsigned long long>(), (unsigned)total, rs.d_ev_temp.p,
+                     rs.d_ev_temp.cap, d_csb, d_csb + sb.cs_begin.size(), rs.cfg.step, rs.cfg.insert_mean + 5 * rs.cfg.insert_std,
+                     rs.d_bad.as<int>(), ctx->sm_count, st, sb.end_bit));
+  ctx->stats.kernel_launches += coverage_launches(sb.end_bit);
+  std::vector<int32_t> bad(std::max<size_t>(n_seg, 1), 0);
+  if (n_seg) CU(cudaMemcpyAsync(bad.data(), rs.d_bad.p, n_seg * 4, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  const int n_cand = (int)sb.n_erased.size();
+  sb.bad.assign(n_cand, 0);
+  for (int c = 0; c < n_cand; c++) {   // bad_bases += added - erased, int arithmetic like the reference
+    int bb = rs.bad_bases;
+    for (int k = 0; k < sb.seg_begin[c + 1] - sb.seg_begin[c]; k++)
+      bb += k < sb.n_erased[c] ? -bad[(size_t)sb.seg_begin[c] + k] : bad[(size_t)sb.seg_begin[c] + k];
+    sb.bad[c] = bb;
+  }
+  sb.imported = true;
+  return GAML_OK;
+}
+
+int gaml_combine_batch_partials(gaml_ctx* ctx, const double* gathered, int32_t n_shards, int32_t n_cand, double* probs,
+                                int32_t* zeros) {
+  if (check_ctx(ctx)) return GAML_ERR_ARG;
+  if (!gathered || !probs || n_shards < 1 || n_cand < 1) return fail(ctx, GAML_ERR_ARG, "bad combine arguments");
+  if (!ctx->shard_batch)
+    return fail(ctx, GAML_ERR_STATE, "gaml_combine_batch_partials: no pending shard batch (call gaml_calc_prob_batch_shard; "
+                                     "any later evaluation, batch or reset drops it)");
+  if (n_cand != (int)ctx->shard_batch_lens.size())
+    return fail(ctx, GAML_ERR_STATE, "gaml_combine_batch_partials: n_cand differs from the pending shard batch's");
+  for (auto& rs : ctx->sets)
+    if (rs->sb.pending && !rs->sb.imported)
+      return fail(ctx, GAML_ERR_STATE, "gaml_combine_batch_partials: a penalised read set's coverage events are not imported yet "
+                                       "(gaml_batch_penalty_export on every shard, then gaml_batch_penalty_import)");
+  const size_t n_sets = ctx->sets.size(), line = n_sets * GAML_PARTIAL_DOUBLES;
+  std::vector<double> one((size_t)n_shards * line);   // one candidate's [n_shards][n_sets][GAML_PARTIAL_DOUBLES]
+  std::vector<int32_t> bad(n_sets);
+  for (int c = 0; c < n_cand; c++) {
+    for (int r = 0; r < n_shards; r++)
+      std::copy_n(gathered + ((size_t)r * n_cand + c) * line, line, one.data() + (size_t)r * line);
+    for (size_t s = 0; s < n_sets; s++) bad[s] = ctx->sets[s]->sb.pending ? ctx->sets[s]->sb.bad[c] : ctx->sets[s]->bad_bases;
+    gaml_result res;
+    const int rc = combine(ctx, one.data(), n_shards, ctx->shard_batch_lens[c], &res, zeros ? zeros + (size_t)c * 2 * n_sets : nullptr,
+                           bad.data());
+    if (rc) return rc;
+    probs[c] = res.prob;
+  }
+  return GAML_OK;
+}
+
 // ---- coverage penalty of a read set on a read-id shard (SURVEY §8f rank 1) --------------------------------------------
 // Paired sets: one 64-bit event key per covered position (walk << 33 | position << 1 | 1, kernels.cu cov_key).
 // PacBio sets: two words per interval {(walk << 32 | start), end}.
@@ -4070,6 +4252,7 @@ int gaml_penalty_import(gaml_ctx* ctx, int set, const uint64_t* all, int64_t n_a
 
 int gaml_reset_state(gaml_ctx* ctx) {
   if (check_ctx(ctx)) return GAML_ERR_ARG;
+  discard_shard_batch(ctx);
   for (auto& rs : ctx->sets) {
     rs->has_state = false;
     rs->total_valid = false;

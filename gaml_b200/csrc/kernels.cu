@@ -13,6 +13,8 @@
 // never carries the general sort/de-dup code through its warps.
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <cub/block/block_scan.cuh>
+#include <cuda/atomic>
 
 #include <chrono>
 #include <cstdio>
@@ -2444,6 +2446,95 @@ __global__ void coverage_sweep_kernel(const unsigned long long* keys, unsigned n
   }
 }
 
+// ---- coverage events of a candidate batch on a read-id shard ------------------------------------------------------
+// A shard exports a thinned subset of its sorted covered-position keys; the sweep of the contig starts plus the union
+// of every shard's subset gives each segment the same bad bases as the sweep of all raw events. Why:
+//  - The sweep adds pos - prev_pos for a covered position only when that gap exceeds `step`. A repeated key sees a gap
+//    of 0 to its copy and a predecessor of the same type, so duplicates in the union change nothing.
+//  - Bucket rule: split a segment's positions into buckets of width w = floor(step) + 1 (w = 1 when step < 0: only
+//    duplicates go), bucket = (segment, u / w) with u = (uint32)(pos ^ 2^31) as in cov_key, and keep only the smallest
+//    and the largest distinct position of each bucket. A dropped p lies strictly between two kept keys k1 < p < k2 of its
+//    bucket, k2 - k1 <= floor(step) <= step. An event e of the union whose predecessor changes by the drop had p or a
+//    later key as predecessor and gets one >= k1; e <= k2 because k2 stays. So e's gap is <= step before and after and e
+//    adds nothing either way; p itself added nothing (p - k1 < step). Every other event keeps its predecessor. The contig
+//    starts come from the host and are in every union, so they are never exported.
+//  - Dropping points one at a time when their two neighbours lie within `step` is NOT exact: with step 10 and positions
+//    0, 8, 10, 18, both inner points pass that test, and dropping both leaves a gap of 18.
+// One thread per kThinItems consecutive sorted keys flags the bucket's first key and the first copy of its last key;
+// the tile's flags are compacted in order by a block scan, and the tiles' offsets chain through a decoupled look-back
+// (state[2 + tile]: 0 = not yet, 1 << 62 = the tile's own count, 2 << 62 = count including every earlier tile). Tiles
+// are numbered by an atomic ticket (state[0]), so a block only ever waits for tiles whose blocks already run.
+constexpr int kThinBlock = 256;
+constexpr int kThinItems = 8;
+constexpr int kThinTile = kThinBlock * kThinItems;
+constexpr unsigned long long kThinOwn = 1ull << 62, kThinAll = 2ull << 62, kThinCount = (1ull << 62) - 1;
+
+__device__ __forceinline__ unsigned long long thin_bucket(unsigned long long k, uint32_t w) {   // w == 0: one bucket
+  const uint32_t u = (uint32_t)(k >> 1);
+  return ((k >> 33) << 32) | (unsigned long long)(w ? u / w : 0u);
+}
+
+__global__ void __launch_bounds__(kThinBlock) coverage_thin_kernel(const unsigned long long* keys, unsigned n, uint32_t w,
+                                                                   unsigned long long* out, unsigned long long* state) {
+  using Scan = cub::BlockScan<unsigned, kThinBlock>;
+  __shared__ typename Scan::TempStorage scan_tmp;
+  __shared__ unsigned long long s_k[kThinTile + 1];   // s_k[1 + t] = keys[base + t], s_k[0] = the key before the tile
+  __shared__ unsigned s_tile;
+  __shared__ unsigned long long s_prefix;
+  if (threadIdx.x == 0) s_tile = (unsigned)atomicAdd(state, 1ull);
+  __syncthreads();
+  const unsigned tile = s_tile;
+  const unsigned base = tile * (unsigned)kThinTile;
+  for (int t = threadIdx.x; t <= kThinTile; t += kThinBlock) {
+    const long long i = (long long)base + t - 1;
+    if (i >= 0 && i < (long long)n) s_k[t] = keys[i];
+  }
+  __syncthreads();
+  auto key_at = [&](unsigned i) { return i - base < (unsigned)kThinTile ? s_k[1 + i - base] : keys[i]; };
+  unsigned mask = 0, count = 0;
+  for (int j = 0; j < kThinItems; j++) {
+    const unsigned t = threadIdx.x * kThinItems + j, i = base + t;
+    if (i >= n) break;
+    const unsigned long long k = s_k[1 + t];
+    bool keep;
+    if (i > 0 && s_k[t] == k) keep = false;                                       // a later copy
+    else if (i == 0 || thin_bucket(s_k[t], w) != thin_bucket(k, w)) keep = true;  // the bucket's smallest position
+    else {                                                                         // its largest: the next key is elsewhere
+      unsigned e = i + 1;
+      while (e < n && key_at(e) == k) e++;
+      keep = e == n || thin_bucket(key_at(e), w) != thin_bucket(k, w);
+    }
+    if (keep) {
+      mask |= 1u << j;
+      count++;
+    }
+  }
+  unsigned offset, aggregate;
+  Scan(scan_tmp).ExclusiveSum(count, offset, aggregate);
+  if (threadIdx.x == 0) {
+    cuda::atomic_ref<unsigned long long, cuda::thread_scope_device> mine(state[2 + tile]);
+    unsigned long long prefix = 0;
+    if (tile > 0) {
+      mine.store(kThinOwn | aggregate, cuda::memory_order_release);
+      for (long long t = (long long)tile - 1; t >= 0; t--) {
+        cuda::atomic_ref<unsigned long long, cuda::thread_scope_device> other(state[2 + t]);
+        unsigned long long s;
+        while (((s = other.load(cuda::memory_order_acquire)) & ~kThinCount) == 0) {
+        }
+        prefix += s & kThinCount;
+        if (s & kThinAll) break;
+      }
+    }
+    mine.store(kThinAll | (prefix + aggregate), cuda::memory_order_release);
+    if ((unsigned long long)base + kThinTile >= n) state[1] = prefix + aggregate;   // the last tile: the kept count
+    s_prefix = prefix;
+  }
+  __syncthreads();
+  unsigned long long o = s_prefix + offset;
+  for (int j = 0; j < kThinItems; j++)
+    if (mask & (1u << j)) out[o++] = s_k[1 + threadIdx.x * kThinItems + j];
+}
+
 // ---- PacBio coverage penalty (CalcScoreForPacbio, graph.cc:3197-3250) --------------------------------------------
 // Per walk the reference sorts interval events — an artificial interval [-1000, 2000), one interval per node, one per
 // alignment at least as probable as its read's minimum (graph.h:478) — and sweeps them with a multiset of open starts;
@@ -3535,6 +3626,22 @@ cudaError_t launch_coverage(const unsigned long long* keys_in, unsigned long lon
   cudaError_t err = cub::DeviceRadixSort::SortKeys(temp, need, keys_in, keys_sorted, (int)n, 0, end_bit, st);
   if (err != cudaSuccess) return err;
   coverage_sweep_kernel<<<grid_for(n, 256, sm_count, 8), 256, 0, st>>>(keys_sorted, n, cs_begin, cs, step, min_from_start, bad);
+  return cudaGetLastError();
+}
+
+size_t coverage_thin_state_bytes(unsigned n) { return (2 + ((size_t)n + kThinTile - 1) / kThinTile) * 8; }
+
+cudaError_t launch_coverage_thin(const unsigned long long* keys_in, unsigned long long* keys_sorted, unsigned n, void* temp,
+                                 size_t temp_bytes, int end_bit, double step, unsigned long long* out, unsigned long long* state,
+                                 cudaStream_t st) {
+  // bucket width floor(step) + 1; 0 stands for 2^32 and more (one bucket per segment); a negative step removes duplicates only
+  const uint32_t w = !(step >= 0) ? 1u : step >= 4294967295.0 ? 0u : (uint32_t)floor(step) + 1u;
+  cudaError_t err = cudaMemsetAsync(state, 0, coverage_thin_state_bytes(n), st);
+  if (err != cudaSuccess || n == 0) return err;
+  size_t need = temp_bytes;
+  err = cub::DeviceRadixSort::SortKeys(temp, need, keys_in, keys_sorted, (int)n, 0, end_bit, st);
+  if (err != cudaSuccess) return err;
+  coverage_thin_kernel<<<(n + kThinTile - 1) / kThinTile, kThinBlock, 0, st>>>(keys_sorted, n, w, out, state);
   return cudaGetLastError();
 }
 

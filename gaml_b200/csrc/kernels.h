@@ -119,6 +119,14 @@ cudaError_t launch_coverage(const unsigned long long* keys_in, unsigned long lon
                             size_t temp_bytes, const int* cs_begin, const int* cs, double step, double min_from_start, int* bad,
                             int sm_count, cudaStream_t st, int end_bit = 64);
 int coverage_launches(int end_bit);   // kernels launch_coverage issues for a sort large enough for CUB's onesweep path
+// A candidate batch's penalised set on a read-id shard: the same radix sort of this shard's covered-position keys, then
+// coverage_thin_kernel keeps the first and last distinct position of every step-wide bucket of each segment, in order,
+// in out (kernels.cu has the argument why the sweep of all shards' kept keys is exact). state: coverage_thin_state_bytes,
+// zeroed here; the kept count is left in state[1]. Issues coverage_launches(end_bit) kernels when n > 0.
+size_t coverage_thin_state_bytes(unsigned n);
+cudaError_t launch_coverage_thin(const unsigned long long* keys_in, unsigned long long* keys_sorted, unsigned n, void* temp,
+                                 size_t temp_bytes, int end_bit, double step, unsigned long long* out, unsigned long long* state,
+                                 cudaStream_t st);
 // PacBio coverage penalty of one set: emit intervals, sort by (walk, start), running max of ends, sort positions, sweep.
 size_t pacbio_coverage_temp_bytes(uint32_t cap);
 cudaError_t launch_pacbio_coverage(const PbCovParams& C, unsigned long long* packed, unsigned long long* run_max, void* temp,

@@ -73,6 +73,44 @@ def sharded_calc_prob(pc, paths: Sequence[Sequence[int]], device=None, gatherer:
     return pc.combine(g, g.shape[0], tl)
 
 
+def allgather_keys(keys: np.ndarray, device=None) -> np.ndarray:
+    """All-gather of a uint64 array whose length differs per rank: the lengths first, then the arrays padded to the
+    longest -> every rank's keys concatenated in rank order (the same array on every rank)."""
+    import torch
+    import torch.distributed as dist
+    keys = np.ascontiguousarray(keys, dtype=np.uint64)
+    if not dist.is_initialized() or dist.get_world_size() == 1:
+        return keys
+    world = dist.get_world_size()
+    dev = device if device is not None else "cpu"
+    n = torch.tensor([len(keys)], dtype=torch.int64, device=dev)
+    ns = [torch.empty_like(n) for _ in range(world)]
+    dist.all_gather(ns, n)
+    ns = [int(x.item()) for x in ns]
+    buf = torch.zeros(max(max(ns), 1), dtype=torch.int64)   # the words as int64: every backend gathers those
+    buf[:len(keys)] = torch.from_numpy(keys.view(np.int64))
+    buf = buf.to(dev)
+    out = [torch.empty_like(buf) for _ in range(world)]
+    dist.all_gather(out, buf)
+    return np.concatenate([o.cpu().numpy()[:k] for o, k in zip(out, ns)]).view(np.uint64)
+
+
+def sharded_calc_prob_batch(pc, packed, device=None):
+    """A candidate batch over all ranks' shards (gaml_calc_prob_batch_shard), penalised paired sets included: this shard's
+    partials and thinned coverage keys -> per penalised set an all-gather of the keys and their import -> all-gather of the
+    partials -> exact combine. Every rank passes the same candidates and gets the same (probs [n], total_lens [n],
+    zeros [n, sets, 2]), bit-identical to an unsharded gaml_calc_prob_batch."""
+    from .workload import KIND_PAIRED
+    part, tls = pc.calc_prob_batch_shard_packed(packed)
+    for s, info in enumerate(pc.sets):
+        spec = info["spec"]
+        if spec.kind == KIND_PAIRED and spec.penalty_constant != 0:
+            pc.batch_penalty_import(s, allgather_keys(pc.batch_penalty_export(s), device))
+    g = allgather_partials(part.reshape(-1), device)
+    probs, zeros = pc.combine_batch_partials(g.reshape((g.shape[0],) + part.shape))
+    return probs, tls, zeros
+
+
 class ResultExchange:
     """Host shared-memory segment for the ranks' 64-byte result lines (gaml_set_result_exchange): rank 0 creates and
     zeroes it, the others attach; `torch.distributed` is used only to hand the name round and as the setup barrier.

@@ -113,6 +113,8 @@ typedef struct {
   int64_t last_batch_cov_events;   /* coverage-gap events (contig starts + covered positions) the last candidate batch sorted and
                                       swept, over its penalised paired sets; 0 without such a set */
   int64_t last_batch_cov_segments; /* coverage segments of that batch: one per (candidate, erased or added walk, penalised set) */
+  int64_t last_batch_cov_exported; /* gaml_calc_prob_batch_shard: the thinned keys it kept for gaml_batch_penalty_export over the
+                                      penalised sets (its last_batch_cov_events count this shard's emitted events); else 0 */
 } gaml_stats;
 
 /* ---- context ---------------------------------------------------------------------------- */
@@ -250,7 +252,7 @@ int gaml_calc_prob_gathered(gaml_ctx* ctx, const int32_t* walk_nodes, const int6
  * added walks', each swept over the current cache: graph.cc:1938, 1946, 1988) on an unsharded context.
  * zeros (optional): n_cand x 2 n_sets. The _partial form returns n_cand x n_sets x GAML_PARTIAL_DOUBLES for shards; it
  * refuses a penalised set (GAML_ERR_UNSUPPORTED): partials carry no bad bases, gaml_combine_partials would apply the
- * base state's. */
+ * base state's. On read-id shards with a penalised set use gaml_calc_prob_batch_shard (below). */
 int gaml_calc_prob_batch(gaml_ctx* ctx, int32_t n_cand, const int32_t* erased_idx, const int64_t* erased_off,
                          const int32_t* added_nodes, const int64_t* added_walk_off, const int64_t* cand_added_off,
                          double* probs, int32_t* total_lens, int32_t* zeros);
@@ -261,10 +263,35 @@ int gaml_calc_prob_batch_partial(gaml_ctx* ctx, int32_t n_cand, const int32_t* e
 /* The multi-GPU form (read-id shards, one context per GPU, every rank calls it with the same candidates): the shards'
  * partials of all candidates are summed by ONE all-reduce on the library's stream (needs gaml_nccl_exchange_init) and
  * combined exactly, so every rank receives the same probs — bit-identical to the unsharded gaml_calc_prob_batch.
- * A penalised set is refused (GAML_ERR_UNSUPPORTED): every candidate's coverage events would have to be all-gathered. */
+ * A penalised set is refused (GAML_ERR_UNSUPPORTED): every candidate's coverage events would have to be all-gathered;
+ * gaml_calc_prob_batch_shard does that with the caller's collective. */
 int gaml_calc_prob_batch_gathered(gaml_ctx* ctx, int32_t n_cand, const int32_t* erased_idx, const int64_t* erased_off,
                                   const int32_t* added_nodes, const int64_t* added_walk_off, const int64_t* cand_added_off,
                                   double* probs, int32_t* total_lens, int32_t* zeros);
+
+/* Candidate batch on read-id shards with penalised paired sets (also unsharded, and without a penalty). A candidate's
+ * bad bases are a sweep over the coverage events of ALL reads, so every rank, with the same candidates:
+ * (1) gaml_calc_prob_batch_shard: the same arguments and outputs as gaml_calc_prob_batch_partial (bit-identical partials
+ *     for an unpenalised set). Per penalised set this shard's events are sorted and thinned on the device: of each
+ *     step-wide bucket of a candidate walk's positions only the first and last distinct position is kept, which leaves
+ *     every walk's sweep unchanged (kernels.cu, coverage_thin_kernel) and the exchange small. Nothing is committed.
+ * (2) per penalised set: gaml_batch_penalty_export (n_out = keys written, or needed when cap is too small), all-gather,
+ *     and gaml_batch_penalty_import with the concatenation of every shard's keys, its own included: the sort and sweep of
+ *     the unsharded batch, giving each candidate bad_bases_c = the state's - the erased walks' + the added walks';
+ * (3) all-gather the partials and gaml_combine_batch_partials(gathered = n_shards x n_cand x n_sets x
+ *     GAML_PARTIAL_DOUBLES, rank-major): probs (and zeros, n_cand x 2 n_sets, optional) bit-identical to an unsharded
+ *     gaml_calc_prob_batch.
+ * The batch stays pending until the next evaluation, batch or gaml_reset_state, which drop it; export, import and combine
+ * then return GAML_ERR_STATE, as do export / import on a set without a penalty and combine before every import or with
+ * another n_cand. gaml_calc_prob_batch_shard returns GAML_ERR_STATE while an evaluation's shard penalty awaits
+ * gaml_penalty_import. */
+int gaml_calc_prob_batch_shard(gaml_ctx* ctx, int32_t n_cand, const int32_t* erased_idx, const int64_t* erased_off,
+                               const int32_t* added_nodes, const int64_t* added_walk_off, const int64_t* cand_added_off,
+                               double* partials, int32_t* total_lens);
+int gaml_batch_penalty_export(gaml_ctx* ctx, int set, uint64_t* out, int64_t cap, int64_t* n_out);
+int gaml_batch_penalty_import(gaml_ctx* ctx, int set, const uint64_t* all, int64_t n_all);
+int gaml_combine_batch_partials(gaml_ctx* ctx, const double* gathered, int32_t n_shards, int32_t n_cand, double* probs,
+                                int32_t* zeros);
 
 /* Coverage-gap penalty (penalty_constant != 0) of a paired or PacBio set on a READ-ID SHARD (SURVEY §8f rank 1): the sweep of
  * graph.cc:1893-1919 / 3197-3250 runs over a walk's events from ALL reads, so after gaml_eval_finish[_gathered] every rank

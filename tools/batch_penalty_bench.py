@@ -5,6 +5,10 @@ Two contexts over the same workload (BASELINE config 2, or one eighth of config 
 one with a penalty on the paired set, both after the same incremental history. The same 1024 candidates
 (bench.make_candidates) are scored by both, alternating, several times. Then the penalised context's sequential
 alternative — calc_prob(candidate) and calc_prob(base) for each of a sample of candidates — scaled to the batch size.
+With --shards N, the penalised set is also split into N read-id shard contexts on the same GPU, run one after the other
+(gaml_calc_prob_batch_shard, the thinned coverage keys exported and imported, gaml_combine_batch_partials): per shard its
+call and device time and its emitted events against its exported keys, the import and combine times, and every prob
+checked against the unsharded penalised batch.
 Last, one profiled batch of each (torch.profiler, CUDA kernels) for the per-kernel split of the added time.
 JSON lines go to stdout and to <out>/batch_penalty_<kind>.jsonl (--out; a new temporary directory by default).
 """
@@ -46,6 +50,7 @@ def main():
     ap.add_argument("--step", type=float, default=300.0 - 30.0)
     ap.add_argument("--out", default=None, help="output directory (default: a new temporary directory)")
     ap.add_argument("--no-profile", action="store_true")
+    ap.add_argument("--shards", type=int, default=0, help="also run the penalised batch on N read-id shard contexts")
     args = ap.parse_args()
     if args.out is None:
         args.out = tempfile.mkdtemp(prefix="batch_penalty_")
@@ -121,6 +126,9 @@ def main():
           "penalised_over_plain_library_call": summary["penalised"]["library_call_ms"]["median"] / summary["plain"]["library_call_ms"]["median"],
           "penalised_over_plain_wall": summary["penalised"]["wall_ms"]["median"] / summary["plain"]["wall_ms"]["median"]})
 
+    if args.shards:
+        sharded_leg(args, wl, base, packed, np.asarray(p_pen), summary["penalised"], emit)
+
     if not args.no_profile:   # a run of its own: per-kernel device time of one batch of each context
         import torch
         from torch.profiler import ProfilerActivity, profile
@@ -140,6 +148,82 @@ def main():
     plain.close()
     pen.close()
     out.close()
+
+
+def sharded_leg(args, wl, base, packed, ref_probs, unsharded, emit):
+    """The penalised batch over args.shards read-id shard contexts of one GPU, run one after the other. A multi-GPU job
+    runs the shards side by side, so besides the sum the record gives the slowest shard of each step (the collectives
+    that move the keys and partials between GPUs are not part of it)."""
+    from gaml_b200 import api
+    n = args.shards
+    shards = [api.ProbCalculator.from_workload(wl, shard_of=(r, n)) for r in range(n)]
+
+    def evaluate(walks):
+        parts = [pc.calc_prob_partial(walks) for pc in shards]
+        if n > 1:
+            union = np.concatenate([pc.penalty_export(0) for pc in shards])
+            for pc in shards:
+                pc.penalty_import(0, union)
+        return shards[0].combine(np.stack([p for p, _ in parts]), n, parts[0][1])
+
+    for walks in wl.evals:
+        evaluate(walks)
+
+    def timed(fn):
+        t0 = time.perf_counter()
+        r = fn()
+        return r, (time.perf_counter() - t0) * 1e3
+
+    def once():
+        rec = {k: [] for k in ("call_ms", "library_call_ms", "device_ms", "events", "exported", "export_ms", "import_ms",
+                               "combine_ms")}
+        parts = []
+        for pc in shards:
+            (part, _), ms = timed(lambda: pc.calc_prob_batch_shard_packed(packed))
+            st = pc.stats()
+            parts.append(part)
+            rec["call_ms"].append(ms)
+            rec["library_call_ms"].append(st.last_prepare_host_us * 1e-3)
+            rec["device_ms"].append(st.last_device_ms)
+            rec["events"].append(int(st.last_batch_cov_events))
+            rec["exported"].append(int(st.last_batch_cov_exported))
+        keys = []
+        for pc in shards:
+            k, ms = timed(lambda: pc.batch_penalty_export(0))
+            keys.append(k)
+            rec["export_ms"].append(ms)
+        union = np.concatenate(keys)
+        for pc in shards:
+            rec["import_ms"].append(timed(lambda: pc.batch_penalty_import(0, union))[1])
+        g = np.stack(parts)
+        probs = None
+        for pc in shards:
+            (probs, _), ms = timed(lambda: pc.combine_batch_partials(g))
+            rec["combine_ms"].append(ms)
+        return probs, rec
+
+    once()   # warm-up
+    recs = []
+    for _ in range(args.reps):
+        probs, rec = once()
+        bad = np.flatnonzero(probs != ref_probs)
+        assert len(bad) == 0, ("sharded probs differ from the unsharded batch", bad[:8])
+        recs.append(rec)
+    per_shard = [{k: spread([r[k][i] for r in recs]) for k in ("call_ms", "library_call_ms", "device_ms")} |
+                 {"events": recs[-1]["events"][i], "exported": recs[-1]["exported"][i]} for i in range(n)]
+    for i, ps in enumerate(per_shard):
+        emit({"what": "shard_batch", "n_shards": n, "shard": i, **ps,
+              "exported_over_events": ps["exported"] / max(ps["events"], 1)})
+    steps = ("call_ms", "export_ms", "import_ms", "combine_ms")
+    slowest = {k: spread([max(r[k]) for r in recs]) for k in steps}
+    total = spread([sum(sum(r[k]) for k in steps) for r in recs])
+    critical = spread([sum(max(r[k]) for k in steps) for r in recs])
+    emit({"what": "sharded_batch", "n_shards": n, "candidates": len(ref_probs), "slowest_shard": slowest,
+          "sum_over_shards_ms": total, "slowest_shard_path_ms": critical,
+          "unsharded_penalised_wall_ms": unsharded["wall_ms"], "unsharded_penalised_library_call_ms": unsharded["library_call_ms"],
+          "events": sum(recs[-1]["events"]), "exported": sum(recs[-1]["exported"]), "probs_bit_identical": True})
+    for pc in shards:
+        pc.close()
 
 
 if __name__ == "__main__":
